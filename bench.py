@@ -16,8 +16,9 @@ on tcgen05 -> policy head -> fused legal-move gather + softmax + value/draw sigm
           input batches larger than L2, `streams_in_flight` batches in flight.
   e2e   : the same step through the host-buffer C-ABI call (nsb_eval_decode_async + nsb_await): pinned host inputs,
           H2D + kernel + D2H inside the timed region; e2e.infer_contract is the unmodified Infer contract (dense logits).
-  --impl reference : the reference's CPU path for its CPU-runnable config (pack + its own Random executor compiled from
-          /root/reference into oracle/_ref + decode) on all host cores.
+  --impl reference : the reference's CPU path for its CPU-runnable config (pack + its own Random executor, compiled into
+          oracle/_ref when the reference's sources are given, else its port + decode) on all host cores.
+  --dump-outputs DIR : after the timed steps, the results of the last step's final batches as DIR/<name>.npy.
 Multi-GPU: one process per GPU (torchrun), independent replicas, weak scaling; NCCL only for the barrier, the
 max-over-ranks of the timed region and the final counter reduction.
 """
@@ -228,6 +229,15 @@ class Workload:
                                self.nb.DECODE_PROBS, None, self.d_legal[j].ptr, self.d_win[j].ptr, self.d_draw[j].ptr,
                                self.d_flag[j].ptr)
 
+    def outputs(self, batches):
+        """What dev_step handed back for the given batch indices, in that order: legal-move probabilities (CSR rows of
+        self.off), win and draw rates, NaN flags.  A batch's buffers hold its result until batch i + n_out is launched."""
+        rows = [(self.d_legal[i % self.n_out].to_host((self.n_moves,), np.float32),
+                 self.d_win[i % self.n_out].to_host((self.B,), np.float32),
+                 self.d_draw[i % self.n_out].to_host((self.B,), np.float32),
+                 self.d_flag[i % self.n_out].to_host((self.B,), np.uint8).astype(np.float32)) for i in batches]
+        return {name: np.stack(col) for name, col in zip(("legal_probs", "win", "draw", "nan_flag"), zip(*rows))}
+
     def free(self):
         for b in [self.d_pool, self.d_off, self.d_idx] + self.d_legal + self.d_win + self.d_draw + self.d_flag:
             b.free()
@@ -332,6 +342,10 @@ def run_b200(args):
     elapsed_ms, per_step, (tw0, tw1) = device_leg(nb, rep, ctx, wl, slots, K * bps, W * bps, step_batches=bps)
     launches = ctx.launch_count() - l0 - W * bps
     clocks = sampler.window(tw0, tw1)
+    # the results of the last step's final batches (at most 64 MiB), taken before the legs below reuse the output buffers
+    end = (W + K) * bps
+    n_dump = max(1, min(wl.n_out, bps, (64 << 20) // (wl.n_moves * 4 + B * 12)))
+    dumped = wl.outputs(range(end - n_dump, end)) if args.dump_outputs and info.rank == 0 else None
     counters, elapsed_max = rep.aggregate({"evals": B * K * bps, "batches": K * bps, "legal_moves": wl.n_moves * K * bps},
                                           elapsed_ms, device=dev_device)
     value = rep.whole_job_rate(counters["evals"], elapsed_max)
@@ -512,6 +526,10 @@ def run_b200(args):
         line["selfplay"] = selfplay
     if info.rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline(synth, B, seconds=args.cpu_seconds)
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     if info.rank == 0:
         print(json.dumps(line), flush=True)
     wl.free()
@@ -724,7 +742,13 @@ def main():
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--selfplay-seconds", type=float, default=6.0)
     ap.add_argument("--small-pool", action="store_true", help="8-batch input pool (profiling runs only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step's final batches (at most 8 and 64 MiB) to DIR/<name>.npy, float32: "
+                         "legal_probs [batches, legal moves], win, draw, nan_flag [batches, batch]; the inputs depend on "
+                         "the arguments only, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     c = CONFIGS[args.config]
     for k_arg, k_cfg in (("batch", "batch"), ("channels", "channels"), ("blocks", "blocks"), ("batches_per_step", "batches_per_step"),
                          ("seed", "seed")):
