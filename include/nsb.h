@@ -61,7 +61,7 @@ typedef struct nsb_feature_bitboard {
  * policy conv1x1(C->27) ; value conv1x1(C->1) -> FC(81->hidden) -> FC(hidden->2) -> sigmoid. */
 typedef struct nsb_net_desc {
     int32_t in_channels;  /* feature planes per position: 86 (SimpleFeatures), 93 (CustomFeaturesV1), <= 96 */
-    int32_t channels;     /* trunk width C (128 or 256)          */
+    int32_t channels;     /* trunk width C (128, 192 or 256)     */
     int32_t blocks;       /* residual blocks (10, 20, 40)        */
     int32_t value_hidden; /* hidden units of the value MLP (256) */
 } nsb_net_desc;

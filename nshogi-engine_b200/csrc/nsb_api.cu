@@ -84,7 +84,7 @@ struct Slot {
 
 struct nsb_ctx {
     int gpu = 0, batch_max = 0, num_sms = 0;
-    int max_pairs = 0;  // co-resident CTA pairs of the 256-channel trunk (0: single-CTA kernel)
+    int max_pairs = 0;  // co-resident CTA pairs of the 192- / 256-channel trunk (0: single-CTA kernel)
     bool use_ts = false;       // 128-channel trunk with the weights fed through tensor memory (trunk_ts.cu)
     bool direct_io = false;    // kernels read / write the caller's page-locked buffers themselves (no copy nodes)
     bool fuse_pack = true;     // packed positions are expanded in the trunk prologue (NSB_FUSE_PACK=0: separate pack kernel)
@@ -205,10 +205,10 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
         set_error("nsb_create: bad arguments (batch_max 1..65535, slots 1..16)");
         return NSB_ERR_INVALID;
     }
-    if ((net->channels != 128 && net->channels != 256) || net->blocks < 1 || net->blocks > 80 ||
+    if ((net->channels != 128 && net->channels != 192 && net->channels != 256) || net->blocks < 1 || net->blocks > 80 ||
         net->in_channels < 1 || net->in_channels > kMaxInChannels || net->value_hidden < 1 ||
         net->value_hidden > kMaxHidden) {
-        set_error("nsb_create: unsupported net (channels 128|256, blocks 1..80, in_channels<=%d, hidden<=%d)",
+        set_error("nsb_create: unsupported net (channels 128|192|256, blocks 1..80, in_channels<=%d, hidden<=%d)",
                   kMaxInChannels, kMaxHidden);
         return NSB_ERR_INVALID;
     }
@@ -229,7 +229,8 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
     int rc = trunk_fused_prepare(net->channels);
     if (rc) return rc;
     int max_pairs = 0;
-    // NSB_TRUNK256=single keeps the one-CTA kernel for A/B measurements (diagnostic build only)
+    // NSB_TRUNK256=single keeps the one-CTA kernel for A/B measurements (diagnostic build only); 192-channel nets
+    // always run on the pair kernel
     const char* t256 = getenv("NSB_TRUNK256");
     const char* t128 = getenv("NSB_TRUNK128");
 #ifndef NSB_DIAG
@@ -238,8 +239,8 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
         return NSB_ERR_INVALID;
     }
 #endif
-    if (net->channels == 256 && !(t256 && strcmp(t256, "single") == 0)) {
-        if ((rc = trunk_pair_prepare(&max_pairs))) return rc;
+    if (net->channels == 192 || (net->channels == 256 && !(t256 && strcmp(t256, "single") == 0))) {
+        if ((rc = trunk_pair_prepare(net->channels, &max_pairs))) return rc;
         if (max_pairs > prop.multiProcessorCount / 2) max_pairs = prop.multiProcessorCount / 2;
     }
     // 128 channels: a context with several slots is a throughput pipeline (batches in flight on
@@ -821,7 +822,9 @@ int nsb_cache_clear(nsb_ctx* c) {
 
 const char* nsb_trunk_kernel_name(nsb_ctx* c) {
     if (!c) return "";
-    if (c->max_pairs > 0) return "trunk_pair_kernel (256 ch, cta_group::2 CTA pair)";
+    if (c->max_pairs > 0)
+        return c->desc.channels == 192 ? "trunk_pair_kernel (192 ch, cta_group::2 CTA pair, Cout halves padded to 128 rows)"
+                                       : "trunk_pair_kernel (256 ch, cta_group::2 CTA pair)";
     if (c->duo_ctas > 0 && c->duo_always) {
         static thread_local char name[96];
         snprintf(name, sizeof name, "trunk_duo_kernel (128 ch, weights via TMEM, %d CTA%s per SM)", c->duo_ctas,

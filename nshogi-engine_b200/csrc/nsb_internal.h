@@ -61,24 +61,29 @@ struct TrunkGeom {
     static_assert(SMEM_BYTES <= 232448, "exceeds 227 KB of shared memory");
 };
 
-// Geometry of the CTA-pair trunk kernel for 256-channel nets (trunk_pair.cu, DESIGN.md §6.2): a
-// cluster of two CTAs owns two positions, CTA r holds position r's activations (all 256 channels)
+// Geometry of the CTA-pair trunk kernel for 192- and 256-channel nets (trunk_pair.cu, DESIGN.md §6.2):
+// a cluster of two CTAs owns two positions, CTA r holds position r's activations (all C channels)
 // and the weight rows of Cout half r; one cta_group::2 MMA (M = 256, N = 192) per K = 16 step.
+// At C = 192 a Cout half is 96 channels: TMEM lanes 0..95 (quadrants 0..2) of each CTA; lanes
+// 96..127 multiply zero weight rows and are never read back.  The K side is exact (3 blocks of 64).
+template <int C_>
 struct PairGeom {
-    static constexpr int C = 256;
-    static constexpr int KCH = C / 8;                     // 32 channel chunks per slot
+    static_assert(C_ == 192 || C_ == 256, "pair trunk width must be 192 or 256");
+    static constexpr int C = C_;
+    static constexpr int KCH = C / 8;                     // channel chunks per slot (24 / 32)
     static constexpr int NCOLS = 96;                      // slots of this CTA's position (last real slot 88)
     static constexpr int NPAIR = 2 * NCOLS;               // UMMA N across the pair
     static constexpr int GUARD = 12;
     static constexpr int SPITCH = (GUARD + NCOLS + 11) | 1;
     static constexpr int BUF_BYTES = ((KCH * SPITCH * 16 + 127) / 128) * 128;
-    static constexpr int XCH = 16;                        // channel chunks of one Cout half
+    static constexpr int XCH = C / 16;                    // channel chunks of one Cout half (12 / 16)
+    static constexpr int QUADS = XCH / 4;                 // TMEM lane quadrants holding real Cout rows (3 / 4)
     static constexpr int XROW = 89 * 16;                  // bytes one bulk push moves per chunk: slots 0..88 (the rest
                                                           // of the 96 are padding that is zero on both sides already)
     static constexpr int XPITCH = (NCOLS + 1) * 16;       // exchange buffer chunk pitch: odd slot count, so that
                                                           // the two chunks of one stmatrix hit different banks
     static constexpr int XBUF_BYTES = XCH * XPITCH;
-    static constexpr int NSTAGES = 5;
+    static constexpr int NSTAGES = C == 256 ? 5 : 7;      // weight ring: as deep as shared memory allows
     static constexpr int KC64 = C / 64;
     static constexpr int TMEM_COLS = 256;
     static constexpr int NBARS = 2 * NSTAGES + 4;         // full[], empty[], act, acc, peer_act, skip
@@ -185,7 +190,7 @@ int trunk_ts_prepare();  // 128-channel trunk with the weights fed through tenso
 int launch_trunk_ts(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s);
 int trunk_duo_prepare(int* ctas_per_sm);  // 128-channel trunk sized for two CTAs per SM (trunk_duo.cu)
 int launch_trunk_duo(const DeviceNet& net, const EvalArgs& a, int num_sms, int ctas_per_sm, cudaStream_t s);
-int trunk_pair_prepare(int* max_pairs);  // same for the CTA-pair kernel; reports co-resident clusters
+int trunk_pair_prepare(int channels, int* max_pairs);  // same for the CTA-pair kernel of that width; reports co-resident clusters
 int launch_trunk_pair(const DeviceNet& net, const EvalArgs& a, int max_pairs, cudaStream_t s);
 int umma_probe(int gpu, int n_cols, int k_elems, int shift_rows, int layout, int iters, float* max_err,
                double* cycles_per_mma);

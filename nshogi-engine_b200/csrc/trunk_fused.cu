@@ -316,8 +316,10 @@ int trunk_fused_prepare(int channels) {
 #else
         e = cudaSuccess;
 #endif
+    else if (channels == 192)  // runs on trunk_pair.cu only; there is no one-CTA 192-channel kernel
+        e = cudaSuccess;
     else {
-        set_error("trunk: unsupported width %d (128 or 256)", channels);
+        set_error("trunk: unsupported width %d (128, 192 or 256)", channels);
         return NSB_ERR_INVALID;
     }
     if (e != cudaSuccess) {

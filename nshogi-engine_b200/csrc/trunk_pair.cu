@@ -1,4 +1,4 @@
-// trunk_pair.cu — the position-stationary trunk for 256-channel nets on a CTA PAIR (sm_100a,
+// trunk_pair.cu — the position-stationary trunk for 192- and 256-channel nets on a CTA PAIR (sm_100a,
 // tcgen05 cta_group::2).  Same contract as trunk_fused.cu (reference src/infer/trt.cc:256-261).
 //
 // Why a pair (DESIGN.md §6.2): with 256 channels one SM's shared memory holds the activations of
@@ -9,7 +9,7 @@
 // D[Cout half r][both positions] in its own TMEM - the same shared-memory bytes now feed twice the
 // math (floor 96 cycles).  The price is an exchange after every layer: CTA r holds Cout half r of
 // the OTHER position's output, which belongs in the peer's activation buffer.  The epilogue writes
-// that part into a 24 KB exchange buffer and the bulk-copy engine pushes it through DSMEM
+// that part into an exchange buffer (24 KB at 256 channels) and the bulk-copy engine pushes it through DSMEM
 // (cp.async.bulk.shared::cluster.shared::cta), completing on the peer's activation barrier.  The
 // skip connection of the foreign half travels the other way, ahead of time, into the same buffer.
 //
@@ -30,9 +30,14 @@ namespace {
 
 constexpr uint32_t kPushBar = 2;  // named barrier: 8 epilogue warps arrive, the push warp (warp 3) waits
 
+// 192 channels (PairGeom<192>): the weight tiles keep 128 rows, of which rows 96..127 are zero, so the
+// MMA is unchanged (M = 256 with a third of each half's rows wasted) while the K side shrinks to 3 blocks
+// of 64.  The epilogue warps of TMEM quadrant 3 then write nothing, but keep arriving on bar_act and
+// kPushBar, so that every barrier count is the same at both widths.
+template <int CW>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 trunk_pair_kernel(const DeviceNet net, const EvalArgs a) {
-    using G = PairGeom;
+    using G = PairGeom<CW>;
     constexpr int C = G::C;
     extern __shared__ uint8_t smem_raw[];
     // the dynamic window starts at the same shared::cta offset in both CTAs, so this alignment
@@ -188,7 +193,7 @@ trunk_pair_kernel(const DeviceNet net, const EvalArgs a) {
     } else if (warp == 3) {
         // ===== push warp: the exchange buffer -> the peer's activation buffer, once per conv layer =====
         // The epilogue warps write the peer position's rows first and arrive on kPushBar without
-        // waiting; this warp then issues the 16 bulk copies (one lane each: a copy costs its issuing
+        // waiting; this warp then issues the XCH bulk copies (one lane each: a copy costs its issuing
         // thread ~290 cycles, tools/bulk_probe.py) while they go on with their own position.
         for (int p = 0; p < my_passes; ++p)
             for (int L = 0; L < NL - 1; ++L) {
@@ -206,8 +211,9 @@ trunk_pair_kernel(const DeviceNet net, const EvalArgs a) {
         // ===== expansion + epilogues + heads =====================================================
         const int et = threadIdx.x - 128;  // 0..255
         const int ew = warp - 4;           // 0..7
-        const int q = ew & 3;              // TMEM lane quadrant (== warp % 4): 32 of my 128 Cout
+        const int q = ew & 3;              // TMEM lane quadrant (== warp % 4): 32 of my C/2 Cout
         const int lbw = ew >> 2;           // the 16-lane block of that quadrant this warp owns (both positions)
+        const bool writer = q < G::QUADS;  // quadrant 3 holds no real Cout rows at 192 channels
         if (stamp && et == 0) eval_timeline(a)[4 * NL + 11] = clock64();
         EpilogueMask<3> realmask;
         realmask.init(0, lane);
@@ -230,7 +236,7 @@ trunk_pair_kernel(const DeviceNet net, const EvalArgs a) {
                 float bias[4];
 #pragma unroll
                 for (int k = 0; k < 4; ++k)
-                    bias[k] = __ldg(net.bias + (size_t)L * C + rank * 128 + q * 32 + 8 * k + (lane >> 2));
+                    bias[k] = writer ? __ldg(net.bias + (size_t)L * C + rank * (C / 2) + q * 32 + 8 * k + (lane >> 2)) : 0.f;
                 mbar_wait(bar_acc, acc_phase);
                 acc_phase ^= 1u;
                 tc_fence_after();
@@ -245,23 +251,25 @@ trunk_pair_kernel(const DeviceNet net, const EvalArgs a) {
                     mbar_wait(bar_skip, skip_phase);
                     skip_phase ^= 1u;
                 }
-                if (residual)
-                    epilogue_half<3, true>(lbw, tq + peer * G::NCOLS, xbuf, G::XPITCH, q * 4, 0, bias, realmask, lane);
-                else
-                    epilogue_half<3, false>(lbw, tq + peer * G::NCOLS, xbuf, G::XPITCH, q * 4, 0, bias, realmask, lane);
+                if (writer) {
+                    if (residual)
+                        epilogue_half<3, true>(lbw, tq + peer * G::NCOLS, xbuf, G::XPITCH, q * 4, 0, bias, realmask, lane);
+                    else
+                        epilogue_half<3, false>(lbw, tq + peer * G::NCOLS, xbuf, G::XPITCH, q * 4, 0, bias, realmask, lane);
+                }
                 fence_proxy_async_smem();
                 named_bar_arrive(kPushBar, kEpiThreads + 32);  // hand the exchange buffer to the push warp, do not wait
                 // then my own position, in place in my activation buffer
-                {
+                if (writer) {
                     const uint32_t out_buf = out_base + G::GUARD * 16;
                     const int chunk0 = (int)rank * G::XCH + q * 4;
                     if (residual)
                         epilogue_half<3, true>(lbw, tq + rank * G::NCOLS, out_buf, G::SPITCH * 16, chunk0, 0, bias, realmask, lane);
                     else
                         epilogue_half<3, false>(lbw, tq + rank * G::NCOLS, out_buf, G::SPITCH * 16, chunk0, 0, bias, realmask, lane);
-                    tc_fence_before();
-                    fence_proxy_async_smem();
                 }
+                tc_fence_before();
+                fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_act);
                 if (stamp && p == 0 && et == 0) eval_timeline(a)[4 * L + 3] = clock64();
@@ -295,11 +303,10 @@ trunk_pair_kernel(const DeviceNet net, const EvalArgs a) {
     }
 }
 
-}  // namespace
-
-int trunk_pair_prepare(int* max_pairs) {
-    cudaError_t e = cudaFuncSetAttribute(trunk_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         PairGeom::SMEM_BYTES);
+template <int CW>
+int pair_prepare(int* max_pairs) {
+    cudaError_t e = cudaFuncSetAttribute(trunk_pair_kernel<CW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         PairGeom<CW>::SMEM_BYTES);
     if (e != cudaSuccess) {
         set_error("trunk pair: cudaFuncSetAttribute failed: %s (is this an sm_100a device?)", cudaGetErrorString(e));
         return NSB_ERR_NO_DEVICE;
@@ -307,9 +314,9 @@ int trunk_pair_prepare(int* max_pairs) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2, 1, 1);
     cfg.blockDim = dim3(kThreads, 1, 1);
-    cfg.dynamicSmemBytes = PairGeom::SMEM_BYTES;
+    cfg.dynamicSmemBytes = PairGeom<CW>::SMEM_BYTES;
     int clusters = 0;
-    e = cudaOccupancyMaxActiveClusters(&clusters, trunk_pair_kernel, &cfg);
+    e = cudaOccupancyMaxActiveClusters(&clusters, trunk_pair_kernel<CW>, &cfg);
     if (e != cudaSuccess || clusters < 1) {
         set_error("trunk pair: no co-resident CTA pairs (%s)", cudaGetErrorString(e));
         return NSB_ERR_NO_DEVICE;
@@ -317,12 +324,27 @@ int trunk_pair_prepare(int* max_pairs) {
     if (max_pairs) *max_pairs = clusters;
     return 0;
 }
+}  // namespace
+
+int trunk_pair_prepare(int channels, int* max_pairs) {
+    if (channels == 256) return pair_prepare<256>(max_pairs);
+    if (channels == 192) return pair_prepare<192>(max_pairs);
+    set_error("trunk pair: unsupported width %d (192 or 256)", channels);
+    return NSB_ERR_INVALID;
+}
 
 int launch_trunk_pair(const DeviceNet& net, const EvalArgs& a, int max_pairs, cudaStream_t s) {
     if (a.n <= 0) return 0;
     const int groups = (a.n + 1) / 2;  // upper bound when the launch works on a miss list
     const int pairs = groups < max_pairs ? groups : max_pairs;
-    trunk_pair_kernel<<<2 * pairs, kThreads, PairGeom::SMEM_BYTES, s>>>(net, a);
+    if (net.channels == 256)
+        trunk_pair_kernel<256><<<2 * pairs, kThreads, PairGeom<256>::SMEM_BYTES, s>>>(net, a);
+    else if (net.channels == 192)
+        trunk_pair_kernel<192><<<2 * pairs, kThreads, PairGeom<192>::SMEM_BYTES, s>>>(net, a);
+    else {
+        set_error("trunk pair: unsupported width %d (192 or 256)", net.channels);
+        return NSB_ERR_INVALID;
+    }
     return 1;
 }
 

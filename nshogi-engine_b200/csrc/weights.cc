@@ -21,8 +21,12 @@ size_t blob_floats(const nsb_net_desc& d) {
            H * 81 + H + 2 * H + 2;
 }
 
+// Output channels per 128-row tile: 128 channels are one tile; 192 and 256 are split into two Cout halves, one per
+// CTA of trunk_pair.cu, and a 96-channel half fills rows 0..95 of its tile (rows 96..127 are zero).
+static inline int cout_halves(int channels) { return channels == 128 ? 1 : 2; }
+
 int stages_per_pass(const nsb_net_desc& d) {
-    const int nhalf = d.channels / 128, kc64 = d.channels / 64;
+    const int nhalf = cout_halves(d.channels), kc64 = d.channels / 64;
     return 9 * (kStemCin / 64) * nhalf + 2 * d.blocks * 9 * kc64 * nhalf + kc64;
 }
 
@@ -90,7 +94,7 @@ static inline size_t tile_index(int j, int row, int e) { return ((size_t)j * 128
 void pack_weights(const nsb_net_desc& d, const float* blob, uint16_t* tiles, float* bias,
                   float* fc1t, float* fc1b, float* fc2, float* fc2b) {
     const int C = d.channels, IN = d.in_channels, H = d.value_hidden, NB = d.blocks;
-    const int nhalf = C / 128, kc64 = C / 64;
+    const int nhalf = cout_halves(C), rows = C / nhalf, kc64 = C / 64;
     const size_t tile_elems = kStageBytes / 2;
     const float* w = blob;
     uint16_t* t = tiles;
@@ -102,10 +106,10 @@ void pack_weights(const nsb_net_desc& d, const float* blob, uint16_t* tiles, flo
                     for (int j = 0; j < 8; ++j)
                         for (int row = 0; row < 128; ++row)
                             for (int e = 0; e < 8; ++e) {
-                                const int co = half * 128 + row, ci = kc * 64 + j * 8 + e;
+                                const int co = half * rows + row, ci = kc * 64 + j * 8 + e;
                                 // the stem: twin channels repeat the weights of the scalar planes (nsb_internal.h)
                                 const int src = stem ? stem_source_channel(ci, cin_real) : (ci < cin_real ? ci : -1);
-                                const float v = src >= 0 ? cw[((size_t)co * cin_real + src) * 9 + tap] : 0.f;
+                                const float v = src >= 0 && row < rows ? cw[((size_t)co * cin_real + src) * 9 + tap] : 0.f;
                                 t[tile_index(j, row, e)] = bf16_bits_rne(v);
                             }
                     t += tile_elems;

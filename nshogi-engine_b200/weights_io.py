@@ -82,6 +82,44 @@ def blob_from_state(state: Mapping[str, object], channels: int, blocks: int, val
     return np.concatenate(out).astype(np.float32)
 
 
+def pad_channels(blob: np.ndarray, desc, channels: int) -> np.ndarray:
+    """The blob of the same net at trunk width `channels` >= desc.channels: the added channels get zero conv weights
+    (as outputs and as inputs), zero biases and zero policy / value-conv weights, so they stay exactly zero through
+    every layer and the net computes what it computed before.  `desc` has the attributes of binding.net_desc."""
+    C, IN, H, NB = desc.channels, desc.in_channels, desc.value_hidden, desc.blocks
+    W = channels
+    if W < C:
+        raise ValueError(f"pad_channels: cannot narrow a {C}-channel net to {W}")
+    blob = np.asarray(blob, dtype=np.float32)
+    out, o = [], 0
+
+    def take(shape):
+        nonlocal o
+        n = int(np.prod(shape))
+        a = blob[o:o + n].reshape(shape)
+        o += n
+        return a
+
+    def padded(a, shape):
+        z = np.zeros(shape, dtype=np.float32)
+        z[tuple(slice(0, s) for s in a.shape)] = a
+        out.append(z.reshape(-1))
+
+    padded(take((C, IN, 3, 3)), (W, IN, 3, 3))
+    padded(take((C,)), (W,))
+    for _ in range(2 * NB):
+        padded(take((C, C, 3, 3)), (W, W, 3, 3))
+        padded(take((C,)), (W,))
+    padded(take((27, C)), (27, W))
+    out.append(take((27,)).reshape(-1))
+    padded(take((C,)), (W,))
+    rest = blob[o:]
+    if rest.size != 1 + H * 81 + H + 2 * H + 2:
+        raise ValueError(f"pad_channels: blob has {blob.size} floats, which does not match the net description")
+    out.append(rest)
+    return np.concatenate(out)
+
+
 def write_nsbw(path: str, blob: np.ndarray, channels: int, blocks: int, value_hidden: int = 256, in_channels: int = 86):
     """File format read by infer::B200::load (host/infer_b200.h): "NSBW", u32 version, i32 channels,
     blocks, hidden, in_channels, then the blob."""
