@@ -91,6 +91,7 @@ struct nsb_ctx {
     int duo_ctas = 0;          // > 0: the two-CTAs-per-SM 128-channel trunk (trunk_duo.cu) is available, co-resident CTAs per SM
     int cluster128 = 1;        // NSB_TRUNK128=mc2 / mc4: trunk_fused.cu in clusters of 2 / 4 CTAs that share the weight stream by multicast
     bool duo_always = false;   // every launch uses it (multi-slot pipeline, or forced); otherwise it is chosen per batch size
+    bool quad = false;         // every launch uses the four-positions-per-CTA 128-channel trunk (trunk_quad.cu)
     nsb::DeviceNet net_duo{};  // the same net with the weight stream in trunk_duo.cu's order (when both kernels are loaded)
     void* d_duo_tiles = nullptr;
     // launch durations (ms) that use_duo() chooses by; calibrated on this device / net at nsb_load_weights
@@ -244,23 +245,27 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
         if (max_pairs > prop.multiProcessorCount / 2) max_pairs = prop.multiProcessorCount / 2;
     }
     // 128 channels: a context with several slots is a throughput pipeline (batches in flight on
-    // several streams) and gets the two-CTAs-per-SM kernel (trunk_duo.cu: +6 % throughput, measured);
+    // several streams) and gets the two-CTAs-per-SM kernel (trunk_duo.cu: +6 % throughput, measured), or with
+    // >= 4 slots the four-positions-per-CTA kernel (trunk_quad.cu: one CTA per SM, so a launch of 256 positions fills
+    // only 64 SMs and it takes about three launches in flight to cover the GPU);
     // a one-slot context evaluates one batch at a time and gets the kernel with the shorter launch
-    // (trunk_fused.cu).  NSB_TRUNK128 = classic | duo | mc2 | mc4 | ts forces one (mc2 / mc4: trunk_fused.cu in clusters that share the
-    // weight stream by multicast; ts: experimental trunk_ts.cu, diagnostic build).
+    // (trunk_fused.cu).  NSB_TRUNK128 = classic | duo | quad | mc2 | mc4 | ts forces one (mc2 / mc4: trunk_fused.cu in clusters
+    // that share the weight stream by multicast; ts: experimental trunk_ts.cu, diagnostic build).
     const bool is128 = net->channels == 128;
     const bool use_ts = is128 && t128 && strcmp(t128, "ts") == 0;
-    // Unforced, a 128-channel context loads BOTH kernels: a multi-slot pipeline always launches the duo kernel; a
+    // Unforced, a 128-channel context loads BOTH kernels: a pipeline of 2-3 slots always launches the duo kernel; a
     // one-slot context picks per batch - trunk_fused.cu while the batch fits one wave of one CTA per SM (shortest
     // launch), trunk_duo.cu (two co-resident CTAs per SM share the tensor pipe) where that is faster (use_duo()).
     const int cluster128 = (is128 && t128 && strcmp(t128, "mc2") == 0) ? 2 : (is128 && t128 && strcmp(t128, "mc4") == 0) ? 4 : 1;
-    const bool want_duo = is128 && !use_ts && (t128 ? strcmp(t128, "duo") == 0 : true);
+    const bool want_quad = is128 && (t128 ? strcmp(t128, "quad") == 0 : slots >= 4);
+    const bool want_duo = is128 && !use_ts && !want_quad && (t128 ? strcmp(t128, "duo") == 0 : true);
     const bool duo_always = want_duo && (t128 ? true : slots >= 2);
 #ifdef NSB_DIAG
     if (use_ts && (rc = trunk_ts_prepare())) return rc;
 #endif
     int duo_ctas = 0;
     if (want_duo && (rc = trunk_duo_prepare(&duo_ctas))) return rc;
+    if (want_quad && (rc = trunk_quad_prepare())) return rc;
     nsb_ctx* c = new (std::nothrow) nsb_ctx();
     if (!c) {
         set_error("out of host memory");
@@ -273,6 +278,7 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
     c->use_ts = use_ts;
     c->duo_ctas = duo_ctas;
     c->duo_always = duo_always;
+    c->quad = want_quad;
     c->cluster128 = cluster128;
     if (const char* dc = getenv("NSB_DUO_CTAS")) c->duo_ctas = duo_ctas > 0 ? atoi(dc) : 0;  // diagnostics: force the grid cap
     if (const char* fp = getenv("NSB_FUSE_PACK")) c->fuse_pack = strcmp(fp, "0") != 0;
@@ -367,10 +373,10 @@ int nsb_load_weights(nsb_ctx* c, const float* blob, size_t n_floats) {
     std::vector<uint16_t> tiles((size_t)stages * kStageBytes / 2);
     std::vector<float> bias((size_t)NL * C), fc1t((size_t)81 * H), fc1b(H), fc2(2 * (size_t)H), fc2b(2);
     pack_weights(d, blob, tiles.data(), bias.data(), fc1t.data(), fc1b.data(), fc2.data(), fc2b.data());
-    const bool ts_only = c->use_ts || (c->duo_ctas > 0 && c->duo_always);
+    const bool ts_only = c->use_ts || c->quad || (c->duo_ctas > 0 && c->duo_always);
     std::vector<uint16_t> ts_tiles;
     int ts_stages = 0;
-    if (c->use_ts || c->duo_ctas > 0) {  // same bias / FC arrays; the conv weights as a stream of 4 KB K = 16 steps
+    if (ts_only || c->duo_ctas > 0) {  // same bias / FC arrays; the conv weights as a stream of 4 KB K = 16 steps
         ts_stages = ts_steps_per_pass(d);
         ts_tiles.assign((size_t)ts_stages * 2048, 0);
         pack_weights_ts(d, blob, ts_tiles.data());
@@ -487,6 +493,7 @@ static int run_trunk(nsb_ctx* c, Slot& s, const EvalArgs& a) {
         NSB_CUDA(cudaEventRecord(s.ev[s.ev_used], s.stream));
     }
     int k = c->max_pairs > 0 ? launch_trunk_pair(c->net, a, c->max_pairs, s.stream)
+            : c->quad        ? launch_trunk_quad(c->net, a, c->num_sms, s.stream)
             : use_duo(c, a.n) ? launch_trunk_duo(c->net_duo, a, c->num_sms, c->duo_ctas, s.stream)
 #ifdef NSB_DIAG
             : c->use_ts      ? launch_trunk_ts(c->net, a, c->num_sms, s.stream)
@@ -825,6 +832,7 @@ const char* nsb_trunk_kernel_name(nsb_ctx* c) {
     if (c->max_pairs > 0)
         return c->desc.channels == 192 ? "trunk_pair_kernel (192 ch, cta_group::2 CTA pair, Cout halves padded to 128 rows)"
                                        : "trunk_pair_kernel (256 ch, cta_group::2 CTA pair)";
+    if (c->quad) return "trunk_quad_kernel (128 ch, 4 positions per CTA, weights via TMEM, 1 CTA per SM)";
     if (c->duo_ctas > 0 && c->duo_always) {
         static thread_local char name[96];
         snprintf(name, sizeof name, "trunk_duo_kernel (128 ch, weights via TMEM, %d CTA%s per SM)", c->duo_ctas,

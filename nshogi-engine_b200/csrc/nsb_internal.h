@@ -190,6 +190,8 @@ int trunk_ts_prepare();  // 128-channel trunk with the weights fed through tenso
 int launch_trunk_ts(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s);
 int trunk_duo_prepare(int* ctas_per_sm);  // 128-channel trunk sized for two CTAs per SM (trunk_duo.cu)
 int launch_trunk_duo(const DeviceNet& net, const EvalArgs& a, int num_sms, int ctas_per_sm, cudaStream_t s);
+int trunk_quad_prepare();  // 128-channel trunk with four positions per CTA, one CTA per SM (trunk_quad.cu)
+int launch_trunk_quad(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s);
 int trunk_pair_prepare(int channels, int* max_pairs);  // same for the CTA-pair kernel of that width; reports co-resident clusters
 int launch_trunk_pair(const DeviceNet& net, const EvalArgs& a, int max_pairs, cudaStream_t s);
 int umma_probe(int gpu, int n_cols, int k_elems, int shift_rows, int layout, int iters, float* max_err,

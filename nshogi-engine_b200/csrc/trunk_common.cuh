@@ -68,10 +68,11 @@ __device__ __forceinline__ int eval_index(const EvalArgs& a, int li, int n_eff) 
 // the 256 epilogue threads (et = 0..255): bitboards -> featS (bit strings) -> 16-byte records
 // [chunk j][slot][8 channels] of the stem's B operand at `stem_buf` (generic pointer to slot 0 of
 // chunk 0 minus the guard, i.e. the buffer base).  `tl` (optional) receives clock64 stamps.
-// NT = number of threads doing the expansion (the kEpiBar named barrier is used with NT threads).
+// NT = number of threads doing the expansion (named barrier `bar` is used with NT threads).
 template <int NPOS, int SPITCH, int GUARD, int NT = kEpiThreads>
 __device__ __forceinline__ void expand_features(const DeviceNet& net, const EvalArgs& a, int n_eff, int li0, uint4* featS,
-                                                uint8_t* stem_buf, int et, unsigned long long* tl) {
+                                                uint8_t* stem_buf, int et, unsigned long long* tl,
+                                                uint32_t bar = kEpiBar) {
     const int IN = net.in_channels, stem_chunks = 2 * net.stem_steps;
     // Per plane: the 81 occupancy bits as one contiguous little-endian bit string with the
     // rotation (extractbit.cu:20,26) already applied, plus the fill value as bf16 bits.
@@ -99,7 +100,7 @@ __device__ __forceinline__ void expand_features(const DeviceNet& net, const Eval
         }
     }
     if (tl) tl[9] = clock64();
-    named_bar_sync(kEpiBar, NT);
+    named_bar_sync(bar, NT);
     if (tl) tl[3] = clock64();
     // The stem reads stem_chunks chunks of 8 input channels: the real ones, the twins of the scalar planes, zero padding
     // (86 + 4 -> 96 channels = 12 chunks; 93 + 11 -> 128 = 16 chunks).  One work
@@ -177,9 +178,10 @@ __device__ __forceinline__ void fc1_prefetch(const DeviceNet& net, int et, float
 // the launch carries a cache, stores the row from its registers - probabilities for NSB_DECODE_PROBS
 // (feedworker.cc:134-135), raw logits for LOGITS / BOTH (frame.cc:110-114), nothing for a row with NaNFound -;
 // then all warps rank the rows (Node::sort) when the request asks for the order.  The caller has passed a
-// kEpiBar barrier after writing scratch / wd and passes one before reusing them.
+// barrier (named barrier `bar` of the NT threads) after writing scratch / wd and passes one before reusing them.
 template <int NPOS, int NT>
-__device__ __forceinline__ void decode_tail(const EvalArgs& a, int n_eff, int li0, float* scratch, const float* wd, int et) {
+__device__ __forceinline__ void decode_tail(const EvalArgs& a, int n_eff, int li0, float* scratch, const float* wd, int et,
+                                            uint32_t bar = kEpiBar) {
     constexpr int NW = NT / 32;
     const int ew = et >> 5, lane = et & 31;
     if (ew < NPOS) {
@@ -209,7 +211,7 @@ __device__ __forceinline__ void decode_tail(const EvalArgs& a, int n_eff, int li
         }
     }
     if (a.order_out != nullptr) {  // rank order of the rows (Node::sort): all epilogue warps share the work
-        named_bar_sync(kEpiBar, NT);
+        named_bar_sync(bar, NT);
         const int pos = ew % NPOS;
         const int b = eval_index(a, li0 + pos, n_eff);
         // the order is staged behind the row's values in the position's (dead) logits scratch
@@ -218,12 +220,77 @@ __device__ __forceinline__ void decode_tail(const EvalArgs& a, int n_eff, int li
             const uint32_t mb = __ldg(a.move_off + b), me = __ldg(a.move_off + b + 1);
             rank_row_coop(scratch + pos * kPolicySize, (int)(me - mb), ew / NPOS, NW / NPOS, lane, ostage);
         }
-        named_bar_sync(kEpiBar, NT);
+        named_bar_sync(bar, NT);
         if (b >= 0) {
             const uint32_t mb = __ldg(a.move_off + b), me = __ldg(a.move_off + b + 1);
             rank_row_copy_out(ostage, (int)(me - mb), ew / NPOS, NW / NPOS, lane, a.order_out + mb);
         }
     }
+}
+
+// K = 16 steps of the TS weight stream (trunk_duo.cu, trunk_quad.cu) per (layer L, K block kc, any tap): the stem's second block holds channels 64..95 (or 64..127) only
+__device__ __forceinline__ int block_steps(const DeviceNet& net, int L, int kc) { return (L == 0 && kc == 1) ? net.stem_steps - 4 : 4; }
+
+// Tail of a pass with NT epilogue threads synchronised on named barrier `bar` (the 256-thread version with its FC1 prefetch is
+// heads_tail below): dense logits, value MLP, sigmoids, fused decode (+ cache store).
+template <int NPOS, int NT>
+__device__ __forceinline__ void heads_tail_small(const DeviceNet& net, const EvalArgs& a, int n_eff, int li0,
+                                                 float* scratch, const float* vbuf, float* red, int et,
+                                                 uint32_t bar = kEpiBar) {
+    constexpr int NW = NT / 32;
+    const int ew = et >> 5, lane = et & 31;
+    const int H = net.hidden;
+    if (a.policy != nullptr) {
+        for (int idx = et; idx < NPOS * kPolicySize; idx += NT) {
+            const int pos = idx / kPolicySize, b = eval_index(a, li0 + pos, n_eff);
+            if (b >= 0) a.policy[(size_t)b * kPolicySize + (idx - pos * kPolicySize)] = scratch[idx];
+        }
+    }
+    float o[NPOS][2];
+#pragma unroll
+    for (int pos = 0; pos < NPOS; ++pos) o[pos][0] = o[pos][1] = 0.f;
+    for (int h = et; h < H; h += NT) {  // FC(81 -> H) + ReLU, folded straight into FC(H -> 2)
+        float acc[NPOS];
+        const float b1 = __ldg(net.fc1b + h);
+#pragma unroll
+        for (int pos = 0; pos < NPOS; ++pos) acc[pos] = b1;
+#pragma unroll 9
+        for (int t = 0; t < 81; ++t) {
+            const float w = __ldg(net.fc1t + (size_t)t * H + h);
+#pragma unroll
+            for (int pos = 0; pos < NPOS; ++pos) acc[pos] += w * vbuf[pos * 81 + t];
+        }
+        const float w0 = __ldg(net.fc2 + h), w1 = __ldg(net.fc2 + H + h);
+#pragma unroll
+        for (int pos = 0; pos < NPOS; ++pos) {
+            const float hid = fmaxf(acc[pos], 0.f);
+            o[pos][0] += w0 * hid;
+            o[pos][1] += w1 * hid;
+        }
+    }
+#pragma unroll
+    for (int pos = 0; pos < NPOS; ++pos)
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            const float s = warp_sum(o[pos][k]);
+            if (lane == 0) red[(ew * NPOS + pos) * 2 + k] = s;
+        }
+    named_bar_sync(bar, NT);
+    if (et < NPOS * 2) {
+        const int pos = et >> 1, k = et & 1;
+        float s = __ldg(net.fc2b + k);
+#pragma unroll
+        for (int qq = 0; qq < NW; ++qq) s += red[(qq * NPOS + pos) * 2 + k];
+        const float val = 1.0f / (1.0f + expf(-s));
+        red[NW * NPOS * 2 + pos * 2 + k] = val;
+        const int b = eval_index(a, li0 + pos, n_eff);
+        if (b >= 0) (k == 0 ? a.win : a.draw)[b] = val;
+    }
+    if (a.move_off != nullptr) {
+        named_bar_sync(bar, NT);
+        decode_tail<NPOS, NT>(a, n_eff, li0, scratch, red + NW * NPOS * 2, et, bar);
+    }
+    named_bar_sync(bar, NT);
 }
 
 // Tail of a pass for the NPOS work-list entries at li0, executed by the 256 epilogue threads after the
