@@ -88,11 +88,11 @@ struct nsb_ctx {
     bool use_ts = false;       // 128-channel trunk with the weights fed through tensor memory (trunk_ts.cu)
     bool direct_io = false;    // kernels read / write the caller's page-locked buffers themselves (no copy nodes)
     bool fuse_pack = true;     // packed positions are expanded in the trunk prologue (NSB_FUSE_PACK=0: separate pack kernel)
-    int duo_ctas = 0;          // > 0: the two-CTAs-per-SM 128-channel trunk (trunk_duo.cu) is available, co-resident CTAs per SM
+    int duo_ctas = 0;          // > 0: the two-CTAs-per-SM 128-channel trunk (trunk_duo_kernel) is available, co-resident CTAs per SM
     int cluster128 = 1;        // NSB_TRUNK128=mc2 / mc4: trunk_fused.cu in clusters of 2 / 4 CTAs that share the weight stream by multicast
     bool duo_always = false;   // every launch uses it (multi-slot pipeline, or forced); otherwise it is chosen per batch size
-    bool quad = false;         // every launch uses the four-positions-per-CTA 128-channel trunk (trunk_quad.cu)
-    nsb::DeviceNet net_duo{};  // the same net with the weight stream in trunk_duo.cu's order (when both kernels are loaded)
+    bool quad = false;         // every launch uses the four-positions-per-CTA 128-channel trunk (trunk_quad_kernel)
+    nsb::DeviceNet net_duo{};  // the same net with the weight stream in trunk_duo_kernel's order (when both kernels are loaded)
     void* d_duo_tiles = nullptr;
     // launch durations (ms) that use_duo() chooses by; calibrated on this device / net at nsb_load_weights
     double t_classic_wave = 0.129, t_duo_single = 0.157, t_duo_pair = 0.215;
@@ -245,8 +245,8 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
         if (max_pairs > prop.multiProcessorCount / 2) max_pairs = prop.multiProcessorCount / 2;
     }
     // 128 channels: a context with several slots is a throughput pipeline (batches in flight on
-    // several streams) and gets the two-CTAs-per-SM kernel (trunk_duo.cu: +6 % throughput, measured), or with
-    // >= 4 slots the four-positions-per-CTA kernel (trunk_quad.cu: one CTA per SM, so a launch of 256 positions fills
+    // several streams) and gets the two-CTAs-per-SM kernel (trunk_duo_kernel: +6 % throughput, measured), or with
+    // >= 4 slots the four-positions-per-CTA kernel (trunk_quad_kernel: one CTA per SM, so a launch of 256 positions fills
     // only 64 SMs and it takes about three launches in flight to cover the GPU);
     // a one-slot context evaluates one batch at a time and gets the kernel with the shorter launch
     // (trunk_fused.cu).  NSB_TRUNK128 = classic | duo | quad | mc2 | mc4 | ts forces one (mc2 / mc4: trunk_fused.cu in clusters
@@ -255,7 +255,7 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
     const bool use_ts = is128 && t128 && strcmp(t128, "ts") == 0;
     // Unforced, a 128-channel context loads BOTH kernels: a pipeline of 2-3 slots always launches the duo kernel; a
     // one-slot context picks per batch - trunk_fused.cu while the batch fits one wave of one CTA per SM (shortest
-    // launch), trunk_duo.cu (two co-resident CTAs per SM share the tensor pipe) where that is faster (use_duo()).
+    // launch), trunk_duo_kernel (two co-resident CTAs per SM share the tensor pipe) where that is faster (use_duo()).
     const int cluster128 = (is128 && t128 && strcmp(t128, "mc2") == 0) ? 2 : (is128 && t128 && strcmp(t128, "mc4") == 0) ? 4 : 1;
     const bool want_quad = is128 && (t128 ? strcmp(t128, "quad") == 0 : slots >= 4);
     const bool want_duo = is128 && !use_ts && !want_quad && (t128 ? strcmp(t128, "duo") == 0 : true);
@@ -426,10 +426,10 @@ int nsb_load_weights(nsb_ctx* c, const float* blob, size_t n_floats) {
 }
 
 // One-slot 128-channel contexts hold both trunk kernels and choose per batch from three launch durations: trunk_fused.cu
-// per wave of one CTA per SM (2 positions each), trunk_duo.cu while at most one CTA per SM is resident, and trunk_duo.cu
-// per wave of two co-resident CTAs per SM.  The durations are measured at nsb_load_weights on this device with this net
-// (calibrate_kernel_choice); the initial values (10 x 128 on a B200 at full clocks) only serve contexts whose batch_max
-// is too small for the choice to exist.
+// per wave of one CTA per SM (2 positions each), trunk_duo_kernel while at most one CTA per SM is resident, and
+// trunk_duo_kernel per wave of two co-resident CTAs per SM.  The durations are measured at nsb_load_weights on this
+// device with this net (calibrate_kernel_choice); the initial values (10 x 128 on a B200 at full clocks) only serve
+// contexts whose batch_max is too small for the choice to exist.
 static bool use_duo(const nsb_ctx* c, int n) {
     if (c->duo_ctas <= 0) return false;
     if (c->duo_always) return true;
@@ -1096,7 +1096,7 @@ static int debug_timeline(nsb_ctx* c, int slot, const nsb_feature_bitboard* d_fe
         set_error("nsb_debug_trunk_timeline: bad arguments or weights not loaded");
         return NSB_ERR_INVALID;
     }
-    // 4 per layer + 16 phase stamps + per CTA {SM id, globaltimer at start, at end} for up to 1,024 CTAs (trunk_duo.cu)
+    // 4 per layer + 16 phase stamps + per CTA {SM id, globaltimer at start, at end} for up to 1,024 CTAs (trunk_tmem.cu)
     const size_t need = (size_t)c->net.num_layers * 4 + 16 + 3 * 1024;
     if (max_stamps < need) {
         set_error("nsb_debug_trunk_timeline: need room for %zu stamps", need);

@@ -188,9 +188,9 @@ int launch_cache_clear(const DeviceCache& c, cudaStream_t s);
 int trunk_fused_prepare(int channels);  // sets max dynamic smem attribute
 int trunk_ts_prepare();  // 128-channel trunk with the weights fed through tensor memory (trunk_ts.cu)
 int launch_trunk_ts(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s);
-int trunk_duo_prepare(int* ctas_per_sm);  // 128-channel trunk sized for two CTAs per SM (trunk_duo.cu)
+int trunk_duo_prepare(int* ctas_per_sm);  // 128-channel trunk sized for two CTAs per SM (trunk_duo_kernel in trunk_tmem.cu)
 int launch_trunk_duo(const DeviceNet& net, const EvalArgs& a, int num_sms, int ctas_per_sm, cudaStream_t s);
-int trunk_quad_prepare();  // 128-channel trunk with four positions per CTA, one CTA per SM (trunk_quad.cu)
+int trunk_quad_prepare();  // 128-channel trunk with four positions per CTA, one CTA per SM (trunk_quad_kernel in trunk_tmem.cu)
 int launch_trunk_quad(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s);
 int trunk_pair_prepare(int channels, int* max_pairs);  // same for the CTA-pair kernel of that width; reports co-resident clusters
 int launch_trunk_pair(const DeviceNet& net, const EvalArgs& a, int max_pairs, cudaStream_t s);

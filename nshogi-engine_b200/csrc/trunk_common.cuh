@@ -228,7 +228,7 @@ __device__ __forceinline__ void decode_tail(const EvalArgs& a, int n_eff, int li
     }
 }
 
-// K = 16 steps of the TS weight stream (trunk_duo.cu, trunk_quad.cu) per (layer L, K block kc, any tap): the stem's second block holds channels 64..95 (or 64..127) only
+// K = 16 steps of the TS weight stream (trunk_tmem.cu) per (layer L, K block kc, any tap): the stem's second block holds channels 64..95 (or 64..127) only
 __device__ __forceinline__ int block_steps(const DeviceNet& net, int L, int kc) { return (L == 0 && kc == 1) ? net.stem_steps - 4 : 4; }
 
 // Tail of a pass with NT epilogue threads synchronised on named barrier `bar` (the 256-thread version with its FC1 prefetch is

@@ -274,7 +274,7 @@ def test_full_size_batch_invariance(nb, orc, synth, monkeypatch, batch, kernel):
     """BASELINE sizes: every position's result is independent of its batch index, of the batch
     size and of which CTA / accumulator column evaluates it (bit-exact), and equals the oracle on
     the distinct positions.  10 x 128 net == config 2.  Bit-exactness holds per trunk kernel; a one-slot context
-    left to itself (kernel None) switches from trunk_fused.cu to trunk_duo.cu with the batch size, and the two
+    left to itself (kernel None) switches from trunk_fused.cu to trunk_duo_kernel with the batch size, and the two
     differ by float rounding (another K order), so that case is held to the oracle tolerance instead."""
     if kernel:
         monkeypatch.setenv("NSB_TRUNK128", kernel)
@@ -295,7 +295,7 @@ def test_full_size_batch_invariance(nb, orc, synth, monkeypatch, batch, kernel):
     if kernel:
         assert np.array_equal(p_big.view(np.uint32), p_small[perm].view(np.uint32))
         assert np.array_equal(w_big, w_small[perm]) and np.array_equal(d_big, d_small[perm])
-    else:  # 16 positions ran on trunk_fused.cu, 4,096 on trunk_duo.cu
+    else:  # 16 positions ran on trunk_fused.cu, 4,096 on trunk_duo_kernel
         assert np.array_equal(p_big[base:].view(np.uint32), p_big[perm[base:]].view(np.uint32))   # invariance inside the batch
         assert np.max(np.abs(p_big - p_small[perm])) < 2 * TOL_LOGIT_VS_BF16_ORACLE
         assert np.max(np.abs(w_big - w_small[perm])) < 2 * TOL_VALUE_VS_BF16_ORACLE
@@ -482,7 +482,7 @@ def test_cluster_multicast_variant_is_bit_identical(nb, orc, synth, monkeypatch,
 
 
 def test_duo_kernel_selected_for_multi_slot_contexts_and_matches(nb, orc, synth, monkeypatch):
-    """A 128-channel ctx with >= 2 slots launches trunk_duo.cu (two CTAs per SM, weights through tensor
+    """A 128-channel ctx with >= 2 slots launches trunk_duo_kernel (two CTAs per SM, weights through tensor
     memory), a one-slot ctx trunk_fused.cu; both agree with the oracle, and with each other within float
     noise (different K order).  1,000 positions: 500 groups over 296 co-resident CTAs, two passes."""
     monkeypatch.delenv("NSB_TRUNK128", raising=False)
@@ -513,7 +513,7 @@ def test_duo_kernel_selected_for_multi_slot_contexts_and_matches(nb, orc, synth,
     n2, p2, w2, l2 = run(2)
     assert n1 == "trunk_fused_kernel<128>" and n2.startswith("trunk_duo_kernel") and "2 CTAs per SM" in n2
     # a one-slot context left to itself holds both kernels and picks by batch size: 1,000 positions = 500 position pairs
-    # are faster as two waves of co-resident CTA pairs (trunk_duo.cu) than as four waves of one CTA per SM
+    # are faster as two waves of co-resident CTA pairs (trunk_duo_kernel) than as four waves of one CTA per SM
     n0, p0, w0, l0 = run(1)
     assert n0.startswith("trunk_fused_kernel<128>") and "trunk_duo_kernel" in n0
     assert np.array_equal(p0.view(np.uint32), p2.view(np.uint32)) and np.array_equal(l0.view(np.uint32), l2.view(np.uint32))

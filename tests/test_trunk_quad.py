@@ -1,7 +1,8 @@
 """trunk_quad_kernel: the 128-channel trunk with four positions per CTA (two groups of two, each with the duo kernel's
 layout) and one CTA per SM, launched by unforced 128-channel contexts with >= 4 slots.
 
-Every accumulator of the quad kernel receives exactly the MMA sequence of trunk_duo_kernel (layer, K block, tap, step,
+Both kernels are instances of one body in csrc/trunk_tmem.cu (one and two position groups per CTA), and every
+accumulator of the quad kernel receives exactly the MMA sequence of trunk_duo_kernel (layer, K block, tap, step,
 same accumulate flags), so the two kernels must agree bit for bit on every output of every entry point; around that,
 the depth tolerances of test_depth_parity.py against the oracle at config 2, batch invariance at B = 4,096, the paths
 that touch the kernel's work list and I/O, and the kernel choice per slot count."""
