@@ -2,9 +2,9 @@
  * nsb_diag.h - diagnostic entry points, exported ONLY by the diagnostic build of the library
  * (nshogi-engine_b200/libnsb_diag.so = the same sources compiled with -DNSB_DIAG).  That build also carries what the
  * product library (libnsb.so, include/nsb.h) leaves out: clock64 stamps inside the trunk kernels (tools/timeline.py,
- * tools/residency.py), the tcgen05 / bulk-copy probes (tools/umma_probe.py, tools/bulk_probe.py), the superseded
- * one-CTA 256-channel kernel (NSB_TRUNK256=single, the bit-for-bit reference of the CTA-pair kernel) and the
- * experimental trunk_ts.cu (NSB_TRUNK128=ts).  Nothing here replaces a reference interface.
+ * tools/residency.py), the tcgen05 / bulk-copy probes (tools/umma_probe.py, tools/bulk_probe.py) and the superseded
+ * one-CTA 256-channel kernel (NSB_TRUNK256=single, the bit-for-bit reference of the CTA-pair kernel).  Nothing here
+ * replaces a reference interface.
  */
 #ifndef NSB_DIAG_H
 #define NSB_DIAG_H

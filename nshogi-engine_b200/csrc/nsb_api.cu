@@ -80,19 +80,25 @@ struct Slot {
     size_t ev_used = 0;
 };
 
+// The trunk kernel(s) a context launches, decided once by nsb_create.
+enum class Trunk {
+    fused,         // trunk_fused_kernel: 128 channels (NSB_TRUNK128=classic), 256 (NSB_TRUNK256=single, diagnostic build)
+    fused_or_duo,  // one-slot 128-channel context: trunk_fused_kernel<128> or trunk_duo_kernel, per batch (use_duo())
+    duo,           // trunk_duo_kernel
+    quad,          // trunk_quad_kernel
+    pair,          // trunk_pair_kernel: 192 and 256 channels
+};
+
 }  // namespace nsb
 
 struct nsb_ctx {
     int gpu = 0, batch_max = 0, num_sms = 0;
-    int max_pairs = 0;  // co-resident CTA pairs of the 192- / 256-channel trunk (0: single-CTA kernel)
-    bool use_ts = false;       // 128-channel trunk with the weights fed through tensor memory (trunk_ts.cu)
+    nsb::Trunk trunk = nsb::Trunk::fused;
+    int max_pairs = 0;         // grid cap of trunk_pair_kernel: co-resident CTA pairs
+    int duo_ctas = 0;          // grid cap of trunk_duo_kernel: co-resident CTAs per SM
     bool direct_io = false;    // kernels read / write the caller's page-locked buffers themselves (no copy nodes)
     bool fuse_pack = true;     // packed positions are expanded in the trunk prologue (NSB_FUSE_PACK=0: separate pack kernel)
-    int duo_ctas = 0;          // > 0: the two-CTAs-per-SM 128-channel trunk (trunk_duo_kernel) is available, co-resident CTAs per SM
-    int cluster128 = 1;        // NSB_TRUNK128=mc2 / mc4: trunk_fused.cu in clusters of 2 / 4 CTAs that share the weight stream by multicast
-    bool duo_always = false;   // every launch uses it (multi-slot pipeline, or forced); otherwise it is chosen per batch size
-    bool quad = false;         // every launch uses the four-positions-per-CTA 128-channel trunk (trunk_quad_kernel)
-    nsb::DeviceNet net_duo{};  // the same net with the weight stream in trunk_duo_kernel's order (when both kernels are loaded)
+    nsb::DeviceNet net_duo{};  // Trunk::fused_or_duo: the same net with the weight stream in trunk_duo_kernel's order
     void* d_duo_tiles = nullptr;
     // launch durations (ms) that use_duo() chooses by; calibrated on this device / net at nsb_load_weights
     double t_classic_wave = 0.129, t_duo_single = 0.157, t_duo_pair = 0.215;
@@ -213,6 +219,24 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
                   kMaxInChannels, kMaxHidden);
         return NSB_ERR_INVALID;
     }
+    // NSB_TRUNK128 / NSB_TRUNK256 force a trunk kernel for A/B measurements.  An unknown value is an error rather than
+    // the default kernel, so that a measurement never runs a kernel other than the one it names.
+    const char* t128 = getenv("NSB_TRUNK128");
+    const char* t256 = getenv("NSB_TRUNK256");
+    if (t128 && strcmp(t128, "classic") != 0 && strcmp(t128, "duo") != 0 && strcmp(t128, "quad") != 0) {
+        set_error("nsb_create: NSB_TRUNK128=\"%s\" (accepted: classic, duo, quad)", t128);
+        return NSB_ERR_INVALID;
+    }
+    if (t256 && strcmp(t256, "single") != 0) {
+        set_error("nsb_create: NSB_TRUNK256=\"%s\" (accepted: single)", t256);
+        return NSB_ERR_INVALID;
+    }
+#ifndef NSB_DIAG
+    if (t256) {
+        set_error("nsb_create: NSB_TRUNK256=single exists in the diagnostic build only (libnsb_diag.so)");
+        return NSB_ERR_INVALID;
+    }
+#endif
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || gpu < 0 || gpu >= ndev) {
         cudaGetLastError();
@@ -227,45 +251,36 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
         return NSB_ERR_NO_DEVICE;
     }
     NSB_CUDA(cudaSetDevice(gpu));
-    int rc = trunk_fused_prepare(net->channels);
+    // 128 channels: a context with several slots is a throughput pipeline (batches in flight on several streams) and
+    // gets the two-CTAs-per-SM kernel (trunk_duo_kernel: +6 % throughput, measured), or with >= 4 slots the
+    // four-positions-per-CTA kernel (trunk_quad_kernel: one CTA per SM, so a launch of 256 positions fills only 64 SMs
+    // and it takes about three launches in flight to cover the GPU).  A one-slot context evaluates one batch at a time
+    // and loads both trunk_fused_kernel<128> and trunk_duo_kernel: per batch it picks trunk_fused_kernel<128> while the
+    // batch fits one wave of one CTA per SM (shortest launch), trunk_duo_kernel (two co-resident CTAs per SM share the
+    // tensor pipe) where that is faster (use_duo()).  192 and 256 channels run on the CTA-pair kernel; NSB_TRUNK256=single
+    // keeps the one-CTA 256-channel kernel, the pair kernel's bit-for-bit reference.
+    Trunk trunk;
+    if (net->channels != 128)
+        trunk = net->channels == 256 && t256 ? Trunk::fused : Trunk::pair;
+    else if (t128)
+        trunk = strcmp(t128, "classic") == 0 ? Trunk::fused : strcmp(t128, "duo") == 0 ? Trunk::duo : Trunk::quad;
+    else
+        trunk = slots >= 4 ? Trunk::quad : slots >= 2 ? Trunk::duo : Trunk::fused_or_duo;
+    int rc = 0, max_pairs = 0, duo_ctas = 0;
+    switch (trunk) {
+        case Trunk::fused: rc = trunk_fused_prepare(net->channels); break;
+        case Trunk::fused_or_duo:
+            rc = trunk_fused_prepare(net->channels);
+            if (!rc) rc = trunk_duo_prepare(&duo_ctas);
+            break;
+        case Trunk::duo: rc = trunk_duo_prepare(&duo_ctas); break;
+        case Trunk::quad: rc = trunk_quad_prepare(); break;
+        case Trunk::pair:
+            rc = trunk_pair_prepare(net->channels, &max_pairs);
+            if (max_pairs > prop.multiProcessorCount / 2) max_pairs = prop.multiProcessorCount / 2;
+            break;
+    }
     if (rc) return rc;
-    int max_pairs = 0;
-    // NSB_TRUNK256=single keeps the one-CTA kernel for A/B measurements (diagnostic build only); 192-channel nets
-    // always run on the pair kernel
-    const char* t256 = getenv("NSB_TRUNK256");
-    const char* t128 = getenv("NSB_TRUNK128");
-#ifndef NSB_DIAG
-    if ((t256 && strcmp(t256, "single") == 0) || (t128 && strcmp(t128, "ts") == 0)) {
-        set_error("nsb_create: NSB_TRUNK256=single / NSB_TRUNK128=ts exist in the diagnostic build only (libnsb_diag.so)");
-        return NSB_ERR_INVALID;
-    }
-#endif
-    if (net->channels == 192 || (net->channels == 256 && !(t256 && strcmp(t256, "single") == 0))) {
-        if ((rc = trunk_pair_prepare(net->channels, &max_pairs))) return rc;
-        if (max_pairs > prop.multiProcessorCount / 2) max_pairs = prop.multiProcessorCount / 2;
-    }
-    // 128 channels: a context with several slots is a throughput pipeline (batches in flight on
-    // several streams) and gets the two-CTAs-per-SM kernel (trunk_duo_kernel: +6 % throughput, measured), or with
-    // >= 4 slots the four-positions-per-CTA kernel (trunk_quad_kernel: one CTA per SM, so a launch of 256 positions fills
-    // only 64 SMs and it takes about three launches in flight to cover the GPU);
-    // a one-slot context evaluates one batch at a time and gets the kernel with the shorter launch
-    // (trunk_fused.cu).  NSB_TRUNK128 = classic | duo | quad | mc2 | mc4 | ts forces one (mc2 / mc4: trunk_fused.cu in clusters
-    // that share the weight stream by multicast; ts: experimental trunk_ts.cu, diagnostic build).
-    const bool is128 = net->channels == 128;
-    const bool use_ts = is128 && t128 && strcmp(t128, "ts") == 0;
-    // Unforced, a 128-channel context loads BOTH kernels: a pipeline of 2-3 slots always launches the duo kernel; a
-    // one-slot context picks per batch - trunk_fused.cu while the batch fits one wave of one CTA per SM (shortest
-    // launch), trunk_duo_kernel (two co-resident CTAs per SM share the tensor pipe) where that is faster (use_duo()).
-    const int cluster128 = (is128 && t128 && strcmp(t128, "mc2") == 0) ? 2 : (is128 && t128 && strcmp(t128, "mc4") == 0) ? 4 : 1;
-    const bool want_quad = is128 && (t128 ? strcmp(t128, "quad") == 0 : slots >= 4);
-    const bool want_duo = is128 && !use_ts && !want_quad && (t128 ? strcmp(t128, "duo") == 0 : true);
-    const bool duo_always = want_duo && (t128 ? true : slots >= 2);
-#ifdef NSB_DIAG
-    if (use_ts && (rc = trunk_ts_prepare())) return rc;
-#endif
-    int duo_ctas = 0;
-    if (want_duo && (rc = trunk_duo_prepare(&duo_ctas))) return rc;
-    if (want_quad && (rc = trunk_quad_prepare())) return rc;
     nsb_ctx* c = new (std::nothrow) nsb_ctx();
     if (!c) {
         set_error("out of host memory");
@@ -274,13 +289,10 @@ int nsb_create(nsb_ctx** out, int gpu, int batch_max, int slots, const nsb_net_d
     c->gpu = gpu;
     c->batch_max = batch_max;
     c->num_sms = prop.multiProcessorCount;
+    c->trunk = trunk;
     c->max_pairs = max_pairs;
-    c->use_ts = use_ts;
     c->duo_ctas = duo_ctas;
-    c->duo_always = duo_always;
-    c->quad = want_quad;
-    c->cluster128 = cluster128;
-    if (const char* dc = getenv("NSB_DUO_CTAS")) c->duo_ctas = duo_ctas > 0 ? atoi(dc) : 0;  // diagnostics: force the grid cap
+    if (const char* dc = getenv("NSB_DUO_CTAS")) c->duo_ctas = atoi(dc) > 1 ? atoi(dc) : 1;  // diagnostics: force the grid cap
     if (const char* fp = getenv("NSB_FUSE_PACK")) c->fuse_pack = strcmp(fp, "0") != 0;
     // A one-slot context is the latency configuration (one batch at a time: every copy node is serial
     // time) and defaults to direct I/O; a multi-slot pipeline overlaps its copies with other batches'
@@ -373,10 +385,11 @@ int nsb_load_weights(nsb_ctx* c, const float* blob, size_t n_floats) {
     std::vector<uint16_t> tiles((size_t)stages * kStageBytes / 2);
     std::vector<float> bias((size_t)NL * C), fc1t((size_t)81 * H), fc1b(H), fc2(2 * (size_t)H), fc2b(2);
     pack_weights(d, blob, tiles.data(), bias.data(), fc1t.data(), fc1b.data(), fc2.data(), fc2b.data());
-    const bool ts_only = c->use_ts || c->quad || (c->duo_ctas > 0 && c->duo_always);
+    const bool ts_only = c->trunk == Trunk::duo || c->trunk == Trunk::quad;
+    const bool both = c->trunk == Trunk::fused_or_duo;  // the TS stream beside the tile stream, as net_duo
     std::vector<uint16_t> ts_tiles;
     int ts_stages = 0;
-    if (ts_only || c->duo_ctas > 0) {  // same bias / FC arrays; the conv weights as a stream of 4 KB K = 16 steps
+    if (ts_only || both) {  // same bias / FC arrays; the conv weights as a stream of 4 KB K = 16 steps
         ts_stages = ts_steps_per_pass(d);
         ts_tiles.assign((size_t)ts_stages * 2048, 0);
         pack_weights_ts(d, blob, ts_tiles.data());
@@ -410,7 +423,7 @@ int nsb_load_weights(nsb_ctx* c, const float* blob, size_t n_floats) {
     n.fc1b = static_cast<const float*>(c->d_weights[3]);
     n.fc2 = static_cast<const float*>(c->d_weights[4]);
     n.fc2b = static_cast<const float*>(c->d_weights[5]);
-    if (c->duo_ctas > 0 && !c->duo_always) {  // both kernels: a second weight stream beside the first
+    if (both) {
         cudaFree(c->d_duo_tiles);
         c->d_duo_tiles = nullptr;
         NSB_CUDA(cudaMalloc(&c->d_duo_tiles, ts_tiles.size() * 2));
@@ -418,8 +431,6 @@ int nsb_load_weights(nsb_ctx* c, const float* blob, size_t n_floats) {
         c->net_duo = n;
         c->net_duo.stages_per_pass = ts_stages;
         c->net_duo.tiles = static_cast<const uint8_t*>(c->d_duo_tiles);
-    } else {
-        c->net_duo = n;
     }
     c->loaded = true;
     return calibrate_kernel_choice(c);
@@ -431,8 +442,6 @@ int nsb_load_weights(nsb_ctx* c, const float* blob, size_t n_floats) {
 // device with this net (calibrate_kernel_choice); the initial values (10 x 128 on a B200 at full clocks) only serve
 // contexts whose batch_max is too small for the choice to exist.
 static bool use_duo(const nsb_ctx* c, int n) {
-    if (c->duo_ctas <= 0) return false;
-    if (c->duo_always) return true;
     const int groups = (n + 1) / 2, sms = c->num_sms;
     const double classic = c->t_classic_wave * ((groups + sms - 1) / sms);
     const int full = groups / (2 * sms), rest = groups % (2 * sms);  // waves of co-resident pairs, then the remainder
@@ -444,7 +453,7 @@ static bool use_duo(const nsb_ctx* c, int n) {
 // launches after a warm-up each, CUDA events on slot 0's stream.  ~12 launches, once per nsb_load_weights.
 static int calibrate_kernel_choice(nsb_ctx* c) {
     const int sms = c->num_sms;
-    if (c->duo_ctas <= 0 || c->duo_always || c->batch_max <= 2 * sms) return 0;  // one wave of trunk_fused.cu: no choice to make
+    if (c->trunk != Trunk::fused_or_duo || c->batch_max <= 2 * sms) return 0;  // one wave of trunk_fused.cu: no choice to make
     Slot& s = c->slots[0];
     const int n_wave = 2 * sms, n_pair = c->batch_max < 4 * sms ? c->batch_max : 4 * sms;
     NSB_CUDA(cudaMemsetAsync(s.d_feat, 0, (size_t)n_pair * c->desc.in_channels * sizeof(nsb_feature_bitboard), s.stream));
@@ -492,13 +501,17 @@ static int run_trunk(nsb_ctx* c, Slot& s, const EvalArgs& a) {
         }
         NSB_CUDA(cudaEventRecord(s.ev[s.ev_used], s.stream));
     }
-    int k = c->max_pairs > 0 ? launch_trunk_pair(c->net, a, c->max_pairs, s.stream)
-            : c->quad        ? launch_trunk_quad(c->net, a, c->num_sms, s.stream)
-            : use_duo(c, a.n) ? launch_trunk_duo(c->net_duo, a, c->num_sms, c->duo_ctas, s.stream)
-#ifdef NSB_DIAG
-            : c->use_ts      ? launch_trunk_ts(c->net, a, c->num_sms, s.stream)
-#endif
-                             : launch_trunk_fused(c->net, a, c->num_sms, s.stream, c->cluster128);
+    int k = 0;
+    switch (c->trunk) {
+        case Trunk::fused: k = launch_trunk_fused(c->net, a, c->num_sms, s.stream); break;
+        case Trunk::fused_or_duo:
+            k = use_duo(c, a.n) ? launch_trunk_duo(c->net_duo, a, c->num_sms, c->duo_ctas, s.stream)
+                                : launch_trunk_fused(c->net, a, c->num_sms, s.stream);
+            break;
+        case Trunk::duo: k = launch_trunk_duo(c->net, a, c->num_sms, c->duo_ctas, s.stream); break;
+        case Trunk::quad: k = launch_trunk_quad(c->net, a, c->num_sms, s.stream); break;
+        case Trunk::pair: k = launch_trunk_pair(c->net, a, c->max_pairs, s.stream); break;
+    }
     if (k < 0) return k;
     NSB_CUDA(cudaGetLastError());
     c->launches += (uint64_t)k;
@@ -829,19 +842,22 @@ int nsb_cache_clear(nsb_ctx* c) {
 
 const char* nsb_trunk_kernel_name(nsb_ctx* c) {
     if (!c) return "";
-    if (c->max_pairs > 0)
-        return c->desc.channels == 192 ? "trunk_pair_kernel (192 ch, cta_group::2 CTA pair, Cout halves padded to 128 rows)"
-                                       : "trunk_pair_kernel (256 ch, cta_group::2 CTA pair)";
-    if (c->quad) return "trunk_quad_kernel (128 ch, 4 positions per CTA, weights via TMEM, 1 CTA per SM)";
-    if (c->duo_ctas > 0 && c->duo_always) {
-        static thread_local char name[96];
-        snprintf(name, sizeof name, "trunk_duo_kernel (128 ch, weights via TMEM, %d CTA%s per SM)", c->duo_ctas,
-                 c->duo_ctas == 1 ? "" : "s");
-        return name;
+    switch (c->trunk) {
+        case Trunk::fused: return c->desc.channels == 128 ? "trunk_fused_kernel<128>" : "trunk_fused_kernel<256>";
+        case Trunk::fused_or_duo:
+            return "trunk_fused_kernel<128> (trunk_duo_kernel for batches where two CTAs per SM are faster)";
+        case Trunk::duo: {
+            static thread_local char name[96];
+            snprintf(name, sizeof name, "trunk_duo_kernel (128 ch, weights via TMEM, %d CTA%s per SM)", c->duo_ctas,
+                     c->duo_ctas == 1 ? "" : "s");
+            return name;
+        }
+        case Trunk::quad: return "trunk_quad_kernel (128 ch, 4 positions per CTA, weights via TMEM, 1 CTA per SM)";
+        case Trunk::pair:
+            return c->desc.channels == 192 ? "trunk_pair_kernel (192 ch, cta_group::2 CTA pair, Cout halves padded to 128 rows)"
+                                           : "trunk_pair_kernel (256 ch, cta_group::2 CTA pair)";
     }
-    if (c->duo_ctas > 0) return "trunk_fused_kernel<128> (trunk_duo_kernel for batches where two CTAs per SM are faster)";
-    if (c->use_ts) return "trunk_ts_kernel (128 ch, weights via TMEM, experimental)";
-    return c->desc.channels == 128 ? "trunk_fused_kernel<128>" : "trunk_fused_kernel<256>";
+    return "";
 }
 
 uint64_t nsb_cache_num_bundles(nsb_ctx* c) { return c ? (uint64_t)c->cache.num_bundles : 0; }

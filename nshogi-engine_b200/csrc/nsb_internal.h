@@ -163,7 +163,7 @@ size_t blob_floats(const nsb_net_desc& d);
 void blob_random(const nsb_net_desc& d, uint64_t seed, float* blob);
 int stages_per_pass(const nsb_net_desc& d);
 int ts_steps_per_pass(const nsb_net_desc& d);
-void pack_weights_ts(const nsb_net_desc& d, const float* blob, uint16_t* stream);  // trunk_ts.cu's weight stream
+void pack_weights_ts(const nsb_net_desc& d, const float* blob, uint16_t* stream);  // weight stream of the trunk_tmem.cu kernels
 // Packs canonical blob -> host images of DeviceNet arrays (tiles as uint16 bf16 bits).
 void pack_weights(const nsb_net_desc& d, const float* blob, uint16_t* tiles, float* bias,
                   float* fc1t, float* fc1b, float* fc2, float* fc2b);
@@ -176,7 +176,7 @@ int launch_pack_positions(const nsb_position* d_pos, size_t n, nsb_feature_bitbo
 int launch_decode(const float* d_policy, const float* d_win, const float* d_draw, size_t n,
                   const uint32_t* d_off, const uint16_t* d_idx, int mode, float* d_out,
                   uint8_t* d_flag, cudaStream_t s, const uint8_t* d_row_flags = nullptr, float* d_logits_out = nullptr);
-int launch_trunk_fused(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s, int cluster = 1);
+int launch_trunk_fused(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s);
 int launch_cache_probe(const DeviceCache& c, const uint64_t* d_hashes, size_t n, const uint32_t* d_off, float* d_legal,
                        float* d_win, float* d_draw, uint8_t* d_hit, uint8_t* d_nan_flag, int* d_miss_idx, int* d_miss_count,
                        cudaStream_t s, uint16_t* d_order = nullptr, int mode = 0, const uint8_t* d_row_flags = nullptr,
@@ -186,8 +186,6 @@ int launch_cache_store(const DeviceCache& c, const uint64_t* d_hashes, size_t n,
                        uint8_t* d_stored, cudaStream_t s);
 int launch_cache_clear(const DeviceCache& c, cudaStream_t s);
 int trunk_fused_prepare(int channels);  // sets max dynamic smem attribute
-int trunk_ts_prepare();  // 128-channel trunk with the weights fed through tensor memory (trunk_ts.cu)
-int launch_trunk_ts(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s);
 int trunk_duo_prepare(int* ctas_per_sm);  // 128-channel trunk sized for two CTAs per SM (trunk_duo_kernel in trunk_tmem.cu)
 int launch_trunk_duo(const DeviceNet& net, const EvalArgs& a, int num_sms, int ctas_per_sm, cudaStream_t s);
 int trunk_quad_prepare();  // 128-channel trunk with four positions per CTA, one CTA per SM (trunk_quad_kernel in trunk_tmem.cu)

@@ -23,20 +23,13 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <atomic>
-
 #include "trunk_common.cuh"
 
 namespace nsb {
 
 namespace {
 
-// CL > 1: the CTAs of a cluster of CL share ONE weight stream.  Every CTA of a launch reads the same tiles in the same
-// order, so CTA r of a cluster fetches slice r of each tile (16 KB / CL) and the bulk-copy engine multicasts it into the
-// ring slot of all CL CTAs: L2 -> SM weight traffic drops to 1 / CL.  A ring slot is free when the MMAs of ALL CL CTAs
-// that read it have retired (the commit arrives on the slot's barrier in every CTA of the cluster), so the CTAs of a
-// cluster run the same number of passes - one that has no positions left runs on empty boards and stores nothing.
-template <int C, int CL = 1>
+template <int C>
 __global__ void __launch_bounds__(kThreads, 1) trunk_fused_kernel(const DeviceNet net, const EvalArgs a) {
     using G = TrunkGeom<C>;
     extern __shared__ uint8_t smem_raw[];
@@ -59,9 +52,7 @@ __global__ void __launch_bounds__(kThreads, 1) trunk_fused_kernel(const DeviceNe
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_eff = eval_count(a);
     const int groups = (n_eff + G::NPOS - 1) / G::NPOS;
-    const uint32_t crank = CL > 1 ? cluster_ctarank() : 0u;
-    const int first = (int)blockIdx.x - (int)crank;  // the cluster's first CTA has the most passes
-    const int my_passes = first < groups ? (groups - first + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+    const int my_passes = (int)blockIdx.x < groups ? (groups - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
     const int NL = net.num_layers;
 
     if (eval_timeline(a) && blockIdx.x == 0 && threadIdx.x == 128) eval_timeline(a)[4 * NL + 0] = clock64();
@@ -71,23 +62,16 @@ __global__ void __launch_bounds__(kThreads, 1) trunk_fused_kernel(const DeviceNe
     if (threadIdx.x == 0) {
         for (int s = 0; s < G::NSTAGES; ++s) {
             mbar_init(bar_full(s), 1);
-            mbar_init(bar_empty(s), CL);  // the commit of every CTA that reads the slot
+            mbar_init(bar_empty(s), 1);
         }
         mbar_init(bar_act, kEpiWarps);  // one arrival per epilogue warp (256 arrivals on one word serialise)
         mbar_init(bar_acc, 1);
         fence_mbar_init();
-        if constexpr (CL > 1) {
-            // In a cluster the READER arms a slot's barrier - here for the first use, afterwards when it frees the slot -
-            // so that a peer's slice can never arrive at a barrier that does not expect it yet.
-            const uint32_t total = (uint32_t)my_passes * (uint32_t)net.stages_per_pass;
-            for (uint32_t s = 0; s < (uint32_t)G::NSTAGES && s < total; ++s) mbar_arrive_expect_tx(bar_full(s), kStageBytes);
-        }
     }
     fence_proxy_async_smem();
     if (warp == 1) tmem_alloc(smem_u32(const_cast<uint32_t*>(tmem_holder)), G::TMEM_COLS);
     tc_fence_before();
     __syncthreads();
-    if constexpr (CL > 1) cluster_sync_all();  // every CTA's barriers exist before a peer multicasts into them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_holder;
     if (eval_timeline(a) && blockIdx.x == 0 && threadIdx.x == 128) eval_timeline(a)[4 * NL + 1] = clock64();
@@ -105,16 +89,9 @@ __global__ void __launch_bounds__(kThreads, 1) trunk_fused_kernel(const DeviceNe
             for (uint32_t t = me; t < total; t += 2) {
                 const uint32_t stage = t % G::NSTAGES, phase = (t / G::NSTAGES) & 1u;
                 mbar_wait(bar_empty(stage), phase ^ 1u);
-                if constexpr (CL == 1) mbar_arrive_expect_tx(bar_full(stage), kStageBytes);
-                if constexpr (CL > 1) {
-                    constexpr uint32_t kSlice = kStageBytes / CL;
-                    bulk_g2s_multicast(ring + stage * kStageBytes + crank * kSlice,
-                                       net.tiles + (size_t)s_in_pass * kStageBytes + crank * kSlice, kSlice, bar_full(stage),
-                                       (uint16_t)((1u << CL) - 1u));
-                } else {
-                    bulk_g2s(ring + stage * kStageBytes, net.tiles + (size_t)s_in_pass * kStageBytes, kStageBytes,
-                             bar_full(stage));
-                }
+                mbar_arrive_expect_tx(bar_full(stage), kStageBytes);
+                bulk_g2s(ring + stage * kStageBytes, net.tiles + (size_t)s_in_pass * kStageBytes, kStageBytes,
+                         bar_full(stage));
                 s_in_pass += 2;
                 if (s_in_pass >= (uint32_t)net.stages_per_pass) s_in_pass -= (uint32_t)net.stages_per_pass;
             }
@@ -125,8 +102,6 @@ __global__ void __launch_bounds__(kThreads, 1) trunk_fused_kernel(const DeviceNe
         constexpr uint32_t idesc = make_idesc_bf16_f32(128, G::NCOLS);
         constexpr uint32_t b_lbo = G::SPITCH * 16;
         uint32_t stage = 0, phase = 0, act_phase = 0;
-        uint32_t tiles_done = 0;
-        const uint32_t tiles_total = (uint32_t)my_passes * (uint32_t)net.stages_per_pass;
         for (int p = 0; p < my_passes; ++p) {
             for (int L = 0; L < NL; ++L) {
                 mbar_wait(bar_act, act_phase);
@@ -156,17 +131,9 @@ __global__ void __launch_bounds__(kThreads, 1) trunk_fused_kernel(const DeviceNe
                                               smem_desc_from(b_lo + (uint32_t)(2 * k * G::SPITCH), 128), idesc,
                                               (uint32_t)((tap | kc | k) != 0));
                                 }
-                                // frees the ring slot when the MMAs retire (CL > 1: in every CTA of the cluster, after
-                                // arming this CTA's barrier for the slot's next tile)
-                                if constexpr (CL > 1) {
-                                    if (tiles_done + G::NSTAGES < tiles_total) mbar_arrive_expect_tx(bar_full(stage), kStageBytes);
-                                    umma_commit_multicast(bar_empty(stage), (uint16_t)((1u << CL) - 1u));
-                                } else {
-                                    umma_commit(bar_empty(stage));
-                                }
+                                umma_commit(bar_empty(stage));  // frees the ring slot when the MMAs retire
                             }
                             __syncwarp();
-                            ++tiles_done;
                             if (++stage == G::NSTAGES) { stage = 0; phase ^= 1u; }
                         }
                     }
@@ -251,75 +218,26 @@ __global__ void __launch_bounds__(kThreads, 1) trunk_fused_kernel(const DeviceNe
     // ---- teardown -------------------------------------------------------------------------------
     tc_fence_before();
     __syncthreads();
-    if constexpr (CL > 1) cluster_sync_all();  // no peer may still multicast into, or arrive on, a CTA that has left
     if (warp == 1) {
         __syncwarp();
         tmem_dealloc(tmem_base, G::TMEM_COLS);
     }
 }
 
-template <int CL>
-int launch_cluster128(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s) {
-    using G = TrunkGeom<128>;
-    const int groups = (a.n + G::NPOS - 1) / G::NPOS;
-    cudaLaunchConfig_t cfg = {};
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = G::SMEM_BYTES;
-    cfg.stream = s;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = CL;
-    attr.val.clusterDim.y = 1;
-    attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    // clusters of CL one-CTA-per-SM blocks the device holds at once (GPC boundaries cost a few SMs); asked once - several
-    // host threads may race to ask, they get the same answer
-    static std::atomic<int> resident_cached{0};
-    int resident = resident_cached.load(std::memory_order_relaxed);
-    if (resident == 0) {
-        cfg.gridDim = dim3((unsigned)(num_sms / CL * CL));
-        int clusters = 0;
-        if (cudaOccupancyMaxActiveClusters(&clusters, trunk_fused_kernel<128, CL>, &cfg) != cudaSuccess || clusters < 1) {
-            set_error("trunk: clusters of %d CTAs do not fit this device", CL);
-            return NSB_ERR_NO_DEVICE;
-        }
-        resident = clusters * CL < num_sms ? clusters * CL : num_sms / CL * CL;
-        resident_cached.store(resident, std::memory_order_relaxed);
-    }
-    int grid = (groups + CL - 1) / CL * CL;
-    if (grid > resident) grid = resident;
-    cfg.gridDim = dim3((unsigned)grid);
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, trunk_fused_kernel<128, CL>, net, a);
-    if (e != cudaSuccess) {
-        set_error("trunk: cluster launch (%d CTAs per cluster) failed: %s", CL, cudaGetErrorString(e));
-        return NSB_ERR_CUDA;
-    }
-    return 1;
-}
-
 }  // namespace
 
 int trunk_fused_prepare(int channels) {
     cudaError_t e;
-    if (channels == 128) {
+    if (channels == 128)
         e = cudaFuncSetAttribute(trunk_fused_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  TrunkGeom<128>::SMEM_BYTES);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(trunk_fused_kernel<128, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkGeom<128>::SMEM_BYTES);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(trunk_fused_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkGeom<128>::SMEM_BYTES);
-    } else if (channels == 256)
 #ifdef NSB_DIAG  // the one-CTA 256-channel kernel: superseded by trunk_pair.cu, kept as its bit-for-bit reference
+    else if (channels == 256)
         e = cudaFuncSetAttribute(trunk_fused_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  TrunkGeom<256>::SMEM_BYTES);
-#else
-        e = cudaSuccess;
 #endif
-    else if (channels == 192)  // runs on trunk_pair.cu only; there is no one-CTA 192-channel kernel
-        e = cudaSuccess;
     else {
-        set_error("trunk: unsupported width %d (128, 192 or 256)", channels);
+        set_error("trunk: no one-CTA kernel for %d channels in this build", channels);
         return NSB_ERR_INVALID;
     }
     if (e != cudaSuccess) {
@@ -329,10 +247,8 @@ int trunk_fused_prepare(int channels) {
     return 0;
 }
 
-int launch_trunk_fused(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s, int cluster) {
+int launch_trunk_fused(const DeviceNet& net, const EvalArgs& a, int num_sms, cudaStream_t s) {
     if (a.n <= 0) return 0;
-    if (net.channels == 128 && cluster == 2) return launch_cluster128<2>(net, a, num_sms, s);
-    if (net.channels == 128 && cluster == 4) return launch_cluster128<4>(net, a, num_sms, s);
     if (net.channels == 128) {
         using G = TrunkGeom<128>;
         const int groups = (a.n + G::NPOS - 1) / G::NPOS;

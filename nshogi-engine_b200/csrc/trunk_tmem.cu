@@ -6,8 +6,8 @@
 // with the next layer inside one CTA did not pay (DESIGN.md §6.1).  Two independent CTAs on the same SM overlap
 // everything for free: while one is in an epilogue (or its prologue / tail) the other one's MMAs own the tensor pipe.
 // What made that impossible was the footprint of a CTA: 229 KB of shared memory (activations + a 96 KB weight ring),
-// all 512 TMEM columns, 64 K registers.  Feeding the weights through tensor memory (trunk_ts.cu: L2 -> registers ->
-// tcgen05.st -> A operand of tcgen05.mma) removes the ring, and the rest is diet.  A group of 2 positions (N = 192:
+// all 512 TMEM columns, 64 K registers.  Feeding the weights through tensor memory (L2 -> registers -> tcgen05.st ->
+// A operand of tcgen05.mma) removes the ring, and the rest is diet.  A group of 2 positions (N = 192:
 // the weight bytes per FLOP that L2 can sustain) owns two activation buffers and one accumulator; a CTA holds NGRP
 // groups and ONE weight stream.
 //

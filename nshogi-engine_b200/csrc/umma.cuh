@@ -82,16 +82,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uin
         : "memory");
 }
 
-// The same copy delivered to the same shared-memory offset - and completing on the mbarrier at the same offset - in
-// every CTA of the cluster whose bit is set in cta_mask.
-__device__ __forceinline__ void bulk_g2s_multicast(uint32_t dst_smem, const void* src, uint32_t bytes, uint32_t bar,
-                                                   uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;"
-        ::"r"(dst_smem), "l"(src), "r"(bytes), "r"(bar), "h"(cta_mask)
-        : "memory");
-}
-
 // ---- TMEM -----------------------------------------------------------------------------------
 // One full warp allocates `ncols` (power of two >= 32) columns; base address lands in smem.
 __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t ncols) {
@@ -126,8 +116,8 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr, uint32_t 
 // so (addr >> 4) needs no mask, and consecutive K steps differ by a constant in the low word only -
 // one integer add per descriptor instead of a shift and two logic ops on the (narrow) uniform datapath.
 __device__ __forceinline__ uint32_t smem_desc_lo(uint32_t smem_addr, uint32_t lbo_bytes) {
-    // matrix-descriptor-encode(x) = (x & 0x3FFFF) >> 4: in a cluster launch the shared-window address of a CTA of rank > 0
-    // carries its rank above bit 18, which must not spill into the LBO field
+    // matrix-descriptor-encode(x) = (x & 0x3FFFF) >> 4: in a cluster launch (trunk_pair_kernel) the shared-window address
+    // of a CTA of rank > 0 carries its rank above bit 18, which must not spill into the LBO field
     return ((smem_addr & 0x3FFFFu) >> 4) | ((lbo_bytes >> 4) << 16);
 }
 __device__ __forceinline__ uint64_t smem_desc_from(uint32_t lo, uint32_t sbo_bytes) {
@@ -167,46 +157,6 @@ __device__ __forceinline__ void tmem_st_32x32b_x8(uint32_t taddr, const uint32_t
     asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
                  "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
                  : "memory");
-}
-// registers -> TMEM: this thread's lane, 32 consecutive 32-bit columns (four K = 16 steps of an A row)
-__device__ __forceinline__ void tmem_st_32x32b_x32(uint32_t taddr, const uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-        ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]),
-          "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]),
-          "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]), "r"(v[24]), "r"(v[25]), "r"(v[26]),
-          "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
-        : "memory");
-}
-// the same straight from eight 16-byte registers quads (no repacking)
-__device__ __forceinline__ void tmem_st_32x32b_x32(uint32_t taddr, const uint4 (&q)[8]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-        ::"r"(taddr), "r"(q[0].x), "r"(q[0].y), "r"(q[0].z), "r"(q[0].w), "r"(q[1].x), "r"(q[1].y), "r"(q[1].z), "r"(q[1].w),
-          "r"(q[2].x), "r"(q[2].y), "r"(q[2].z), "r"(q[2].w), "r"(q[3].x), "r"(q[3].y), "r"(q[3].z), "r"(q[3].w),
-          "r"(q[4].x), "r"(q[4].y), "r"(q[4].z), "r"(q[4].w), "r"(q[5].x), "r"(q[5].y), "r"(q[5].z), "r"(q[5].w),
-          "r"(q[6].x), "r"(q[6].y), "r"(q[6].z), "r"(q[6].w), "r"(q[7].x), "r"(q[7].y), "r"(q[7].z), "r"(q[7].w)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st_32x32b_x16(uint32_t taddr, const uint4 (&q)[8]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-        ::"r"(taddr), "r"(q[0].x), "r"(q[0].y), "r"(q[0].z), "r"(q[0].w), "r"(q[1].x), "r"(q[1].y), "r"(q[1].z), "r"(q[1].w),
-          "r"(q[2].x), "r"(q[2].y), "r"(q[2].z), "r"(q[2].w), "r"(q[3].x), "r"(q[3].y), "r"(q[3].z), "r"(q[3].w)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st_32x32b_x16(uint32_t taddr, const uint32_t* v) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-        ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]),
-          "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
-        : "memory");
 }
 // Warpgroup register reallocation: every warp of a group of 4 consecutive warps executes it.
 template <int N>
@@ -267,11 +217,6 @@ __device__ __forceinline__ void ldmatrix_x4_trans(uint32_t addr, uint32_t& r0, u
                  : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3)
                  : "r"(addr)
                  : "memory");
-}
-__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
-    uint32_t d;
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
-    return d;
 }
 // ReLU fused into the conversion: negative inputs (and NaN) become +0.
 __device__ __forceinline__ uint32_t pack_relu_bf16x2(float lo, float hi) {
@@ -367,32 +312,11 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t d_tmem, uint64_t a_desc,
         ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// arrive (once) on the mbarrier at this offset in every CTA of `cta_mask` when all MMAs issued so
-// far by this thread have retired
-__device__ __forceinline__ void umma_commit_multicast(uint32_t bar, uint16_t cta_mask) {  // MMAs of cta_group::1
-    asm volatile(
-        "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-        ::"r"(bar), "h"(cta_mask)
-        : "memory");
-}
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t cta_mask) {
     asm volatile(
         "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
         ::"r"(bar), "h"(cta_mask)
         : "memory");
-}
-// packed bf16 pairs <-> TMEM in the 16x128b fragment (thread t: lanes t/4 and t/4+8, column t%4 of
-// each 4-column group) == the C fragment after pairing adjacent columns
-__device__ __forceinline__ void tmem_st_16x128b_x4(uint32_t taddr, const uint32_t (&v)[8]) {
-    asm volatile("tcgen05.st.sync.aligned.16x128b.x4.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
-                 "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-                 : "memory");
-}
-__device__ __forceinline__ void tmem_ld_16x128b_x4(uint32_t taddr, uint32_t (&v)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.16x128b.x4.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-                 : "r"(taddr)
-                 : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() {
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
@@ -400,9 +324,6 @@ __device__ __forceinline__ void tmem_st_wait() {
 
 __device__ __forceinline__ uint16_t f32_to_bf16_bits(float f) {
     return __bfloat16_as_ushort(__float2bfloat16_rn(f));
-}
-__device__ __forceinline__ float bf16_bits_to_f32(uint16_t b) {
-    return __uint_as_float((uint32_t)b << 16);
 }
 
 }  // namespace nsb

@@ -162,7 +162,7 @@ void pack_weights(const nsb_net_desc& d, const float* blob, uint16_t* tiles, flo
 }
 
 
-// ---- "TS" weight stream (trunk_ts.cu: the A operand goes global -> registers -> tensor memory) ------
+// ---- "TS" weight stream (trunk_tmem.cu: the A operand goes global -> registers -> tensor memory) ----
 // One 4 KB block per K = 16 MMA step, [128 accumulator rows][16 input channels] bf16 (a row's 32
 // bytes are exactly what one producer thread stores into its TMEM lane), in issue order:
 //   layer, K block kc (64 input channels; the previous epilogue finishes them in this order),

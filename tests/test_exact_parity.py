@@ -388,13 +388,16 @@ SIZES = (1, 3, 5, 601)   # idle slots in the last group / pair / quad, and a sec
 TOL_PROBS_REL = 2.0 ** -18
 
 # kernel -> (NSB_TRUNK128, NSB_TRUNK256, slots, diag, trunk_kernel_name (the fused kernels' exactly, else its prefix), nets)
+# The *_1slot rows are the kernel choices of one-slot 128-channel contexts: the duo and quad kernels forced, and unforced,
+# where each batch runs on trunk_fused_kernel<128> or trunk_duo_kernel (two weight streams, chosen by batch size).
 KERNELS = {
     "classic": ("classic", None, 1, False, "trunk_fused_kernel<128>", ["128x2", "128x10", "128x2c93"]),
     "duo": (None, None, 2, False, "trunk_duo_kernel", ["128x2", "128x10"]),
     "quad": (None, None, 4, False, "trunk_quad_kernel", ["128x2", "128x10", "128x2c93"]),
-    "mc2": ("mc2", None, 1, False, "trunk_fused_kernel<128>", ["128x2", "128x10"]),
-    "mc4": ("mc4", None, 1, False, "trunk_fused_kernel<128>", ["128x2", "128x10"]),
-    "ts": ("ts", None, 1, True, "trunk_ts_kernel", ["128x2", "128x10"]),
+    "duo_1slot": ("duo", None, 1, False, "trunk_duo_kernel", ["128x2", "128x10"]),
+    "quad_1slot": ("quad", None, 1, False, "trunk_quad_kernel", ["128x2", "128x10"]),
+    "auto_1slot": (None, None, 1, False,
+                   "trunk_fused_kernel<128> (trunk_duo_kernel for batches where two CTAs per SM are faster)", ["128x2", "128x10"]),
     "pair": (None, None, 1, False, "trunk_pair_kernel", ["256x2", "256x10", "192x2", "192x10", "256x2c93"]),
     "single256": (None, "single", 1, True, "trunk_fused_kernel<256>", ["256x2", "256x10"]),
 }

@@ -407,80 +407,6 @@ def test_pair_kernel_stress_over_streams():
     assert "mismatching launches: 0" in out.stdout
 
 
-def test_ts_kernel_matches_oracle_and_default_kernel(nb, orc, synth, monkeypatch):
-    """trunk_ts.cu (NSB_TRUNK128=ts: weights through tensor memory, A operand of tcgen05.mma read from
-    TMEM, K-block-pipelined layers): same results as the oracle within the logit tolerance and the same
-    decoded probabilities as the default kernel within float noise (the K order differs)."""
-    desc = nb.net_desc(128, 4)
-    blob = nb.random_blob(desc, 77)
-    n = 301                                                  # 151 groups over 148 CTAs: two passes on some
-    pos = synth.random_positions(n, seed=12)
-    fb = orc.pack(pos)
-    off, idx = synth.random_legal_moves(n, seed=6, edge_rows=False)
-
-    def run(ts):
-        if ts:
-            monkeypatch.setenv("NSB_TRUNK128", "ts")
-        else:
-            monkeypatch.delenv("NSB_TRUNK128", raising=False)
-        policy = np.zeros((n, nb.POLICY_SIZE), dtype=np.float32)
-        win, draw = np.zeros(n, dtype=np.float32), np.zeros(n, dtype=np.float32)
-        legal = np.zeros(int(off[-1]), dtype=np.float32)
-        with nb.Context(desc, batch_max=n, blob=blob, diag=ts) as ctx:   # trunk_ts.cu: libnsb_diag.so
-            ctx.eval_async(0, fb, n, policy, win, draw)
-            ctx.await_(0)
-            ctx.eval_decode_async(0, fb, n, off, idx, nb.DECODE_PROBS, legal, win, draw, None)
-            ctx.await_(0)
-        return policy, win, draw, legal
-
-    p_ts, w_ts, d_ts, l_ts = run(True)
-    p_df, w_df, d_df, l_df = run(False)
-    op, ow, od = orc.forward(desc, blob, orc.expand(fb[:32 * 86], 32), emulate_bf16=True)
-    assert np.max(np.abs(p_ts[:32] - op)) < 2 * TOL_LOGIT_VS_BF16_ORACLE
-    assert np.max(np.abs(w_ts[:32] - ow)) < 2 * TOL_VALUE_VS_BF16_ORACLE
-    assert np.max(np.abs(l_ts - l_df)) < 5e-3 and np.max(np.abs(w_ts - w_df)) < 2e-3
-
-
-@pytest.mark.parametrize("mode", ["mc2", "mc4"])
-def test_cluster_multicast_variant_is_bit_identical(nb, orc, synth, monkeypatch, mode):
-    """NSB_TRUNK128=mc2 / mc4: trunk_fused.cu in clusters of 2 / 4 CTAs that share ONE weight stream (CTA r fetches slice
-    r of every tile, the bulk-copy engine multicasts it into all ring slots; a slot is free when every CTA's MMAs have
-    retired).  Same arithmetic in the same order: outputs bit-identical to the un-clustered kernel for every batch size
-    - odd sizes, sizes that leave cluster CTAs without positions, several passes - and on REPEATED launches (the
-    UMMA descriptors of a CTA of rank > 0 must not carry the rank bits of its shared-window address)."""
-    desc = nb.net_desc(128, 3)
-    blob = nb.random_blob(desc, 77)
-    sizes = [1, 2, 3, 5, 8, 64, 255, 300, 700]
-    nmax = max(sizes)
-    fb = orc.pack(synth.random_positions(nmax, seed=12))
-    off, idx = synth.random_legal_moves(nmax, seed=13, edge_rows=True)
-
-    def run(force):
-        monkeypatch.setenv("NSB_TRUNK128", force)
-        out = {}
-        with nb.Context(desc, batch_max=nmax, slots=2, blob=blob) as ctx:
-            assert ctx.trunk_kernel_name() == "trunk_fused_kernel<128>"
-            for rep in range(2):
-                for n in sizes:
-                    policy = np.zeros((n, nb.POLICY_SIZE), dtype=np.float32)
-                    win, draw = np.zeros(n, dtype=np.float32), np.zeros(n, dtype=np.float32)
-                    ctx.eval_async(rep, fb[:n], n, policy, win, draw)
-                    ctx.await_(rep)
-                    o = off[: n + 1]
-                    legal = np.zeros(int(o[-1]), dtype=np.float32)
-                    w2, d2 = np.zeros(n, dtype=np.float32), np.zeros(n, dtype=np.float32)
-                    ctx.eval_decode_async(rep, fb[:n], n, o, idx[: int(o[-1])], nb.DECODE_PROBS, legal, w2, d2, None)
-                    ctx.await_(rep)
-                    out[(rep, n)] = (policy, win, draw, legal, w2)
-        return out
-
-    ref, got = run("classic"), run(mode)
-    for key in ref:
-        for a, b in zip(ref[key], got[key]):
-            assert np.array_equal(a, b, equal_nan=True), (mode, key)
-    assert not np.isnan(got[(1, 300)][0]).any()
-
-
 def test_duo_kernel_selected_for_multi_slot_contexts_and_matches(nb, orc, synth, monkeypatch):
     """A 128-channel ctx with >= 2 slots launches trunk_duo_kernel (two CTAs per SM, weights through tensor
     memory), a one-slot ctx trunk_fused.cu; both agree with the oracle, and with each other within float

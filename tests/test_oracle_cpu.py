@@ -276,6 +276,9 @@ def test_library_is_sm100a_tcgen05_and_has_no_oracle(nb):
         # probes, the experimental trunk_ts.cu and the superseded one-CTA 256-channel kernel are not in the product
         kernels = set(re.findall(r"Function : (\S+)", sass.stdout))
         assert kernels and not any(k for k in kernels if "umma_probe" in k or "bulk_" in k or "trunk_ts" in k or "trunk_fused_kernelILi256" in k), kernels
+        # one 128-channel one-CTA kernel, with no cluster-size template argument
+        assert len([k for k in kernels if "trunk_fused_kernelILi128E" in k]) == 1, kernels
+        assert not any("trunk_fused_kernelILi128ELi" in k for k in kernels), kernels
         assert any("trunk_duo_kernel" in k for k in kernels) and any("trunk_pair_kernel" in k for k in kernels)
     needed = subprocess.check_output(["readelf", "-d", nb.LIB_PATH], text=True)
     assert "oracle" not in needed
@@ -298,7 +301,7 @@ def test_fails_loudly_without_gpu(nb):
     assert "-3" in str(e.value) and "no CPU fallback" in str(e.value)
 
 
-def test_create_rejects_bad_arguments(nb):
+def test_create_rejects_bad_arguments(nb, monkeypatch):
     l = nb.lib()
     h = ctypes.c_void_p()
     bad = nb.net_desc(96, 1)
@@ -306,4 +309,16 @@ def test_create_rejects_bad_arguments(nb):
     good = nb.net_desc(128, 1)
     assert l.nsb_create(ctypes.byref(h), 0, 0, 1, ctypes.byref(good)) == -1
     assert l.nsb_create(ctypes.byref(h), 0, 8, 0, ctypes.byref(good)) == -1
+    # an unknown kernel override fails before any device query instead of running some other kernel
+    monkeypatch.delenv("NSB_TRUNK256", raising=False)
+    for value in ("mc2", "mc4", "ts", "bogus", ""):
+        monkeypatch.setenv("NSB_TRUNK128", value)
+        assert l.nsb_create(ctypes.byref(h), 0, 8, 1, ctypes.byref(good)) == -1, value
+        err = l.nsb_last_error()
+        assert b"NSB_TRUNK128" in err and b"classic" in err and b"duo" in err and b"quad" in err, err
+    monkeypatch.delenv("NSB_TRUNK128")
+    monkeypatch.setenv("NSB_TRUNK256", "bogus")
+    assert l.nsb_create(ctypes.byref(h), 0, 8, 1, ctypes.byref(nb.net_desc(256, 1))) == -1
+    err = l.nsb_last_error()
+    assert b"NSB_TRUNK256" in err and b"single" in err, err
     assert l.nsb_await(None, 0) == -1 and b"null ctx" in l.nsb_last_error()

@@ -60,10 +60,8 @@ def main():
     args = ap.parse_args()
     steps = max(20, int(args.seconds / 0.053))
     out = {"one_cta_kernel": bench_line({"NSB_TRUNK128": "classic"}, steps), "duo_kernel": bench_line({"NSB_TRUNK128": "duo"}, steps),
-           "one_cta_kernel_clusters_of_2": bench_line({"NSB_TRUNK128": "mc2"}, steps),
-           "one_cta_kernel_clusters_of_4": bench_line({"NSB_TRUNK128": "mc4"}, steps),
            "cublas": matmul_energy(args.seconds)}
-    for k in ("one_cta_kernel", "duo_kernel", "one_cta_kernel_clusters_of_2", "one_cta_kernel_clusters_of_4"):
+    for k in ("one_cta_kernel", "duo_kernel"):
         e = out[k].get("energy")
         if e:
             e["pj_per_executed_flop"] = round(e["pj_per_useful_flop"] * 162.0 / 192.0, 4)
